@@ -2,6 +2,7 @@
 """bench.py -- env-steps/sec of the fused step kernel (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--env ID] [--log2-envs k]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): CartPole-v1, num_envs = 2^20 per GPU, random int64 actions resident in
 HBM, fused step + TimeLimit + autoreset; a "step" is one vector step of the whole batch (one kernel launch per GPU).
@@ -23,6 +24,12 @@ Prints ONE JSON line (rank 0).  Keys beyond the base contract:
                        MountainCar-v0 at 2^18 envs, LunarLander-v2 / BipedalWalker-v3 at 2^16
   gather_verified      (N>1) every rank checks, per peer, a checksum of that peer's rows in ITS gathered copy
                        against the checksum the peer computed over its own rows
+
+--dump-outputs DIR (N=1, --impl b200) writes what the last timed step returned as DIR/<name>.npy: obs, reward, terminated,
+truncated (0/1) and final_observation (zero where the env did not finish), float32 or float64.  Above 64 MB in all,
+the same seeded sample of env rows is taken from every array and its indices are written as rows.npy.  The inputs
+(reset seed, action generator seed) are fixed, so two builds run with the same arguments can be compared output for
+output.
 """
 import argparse
 import json
@@ -66,6 +73,7 @@ BOUND = {"CartPole-v1": "hbm", "CartPole-v0": "hbm", "Pendulum-v1": "hbm (latenc
 # dram__bytes_read.sum + dram__bytes_write.sum per launch from the committed ncu --set full capture (2^20 envs)
 NCU_DRAM = {"file": "profiles/r2b_cartpole_step_kernel_L_40reg_ncu_full.txt", "read": 52.76e6, "write": 22.86e6}
 FALLBACK_HBM_GBS = 6650.0  # /opt/skills/guides/B200_PROFILING.md fallback
+DUMP_LIMIT_BYTES = 64 << 20
 EXTRA_CONFIGS = [("Pendulum-v1", 18, 300), ("Acrobot-v1", 18, 300), ("MountainCar-v0", 18, 300),
                  ("LunarLander-v2", 16, 150), ("BipedalWalker-v3", 16, 60)]
 
@@ -73,7 +81,7 @@ EXTRA_CONFIGS = [("Pendulum-v1", 18, 300), ("Acrobot-v1", 18, 300), ("MountainCa
 def parse_args():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=1000)
+    p.add_argument("--steps", type=int, default=1000, help="timed steps (>= 1)")
     p.add_argument("--warmup", type=int, default=100)
     p.add_argument("--impl", default="b200", choices=["b200", "reference"])
     p.add_argument("--env", default=ENV_ID)
@@ -86,7 +94,15 @@ def parse_args():
     p.add_argument("--no-extra", action="store_true", help="skip the configs[2]/[3] lines and the strong-scaling run")
     p.add_argument("--gather", default="p2p", choices=["p2p", "nccl"],
                    help="N>1 exchange: fused NVLink peer pushes in the step kernel, or NCCL all-gather")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and (args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        p.error("--dump-outputs takes --gpus 1 and a single process")
+    if args.dump_outputs and args.impl != "b200":
+        p.error("--dump-outputs dumps the B200 path's outputs: it takes --impl b200")
+    return args
 
 
 # --------------------------------------------------------------------------- helpers
@@ -264,17 +280,10 @@ def run_reference(args):
     pool = [random_actions_np(args.env, n, rng) for _ in range(4)]
     for w in range(max(args.warmup, 1)):
         v.step(pool[w % 4], nthreads=threads)
-        if w >= 5:
-            break
-    steps = min(args.steps, 2000)
-    # bounded sample: stop after ~60 s even if K steps are not through
+    done = args.steps
     t0 = time.perf_counter()
-    done = 0
-    for k in range(steps):
+    for k in range(done):
         v.step(pool[k % 4], nthreads=threads)
-        done += 1
-        if time.perf_counter() - t0 > 60.0 and done >= 3:
-            break
     el = time.perf_counter() - t0
     v.close()
     value = n * done / el
@@ -320,17 +329,41 @@ class L2Flush:
 
 
 def time_steps_flushed(torch, env, pool, K, flush):
-    """K steps, L2 flushed before each, one CUDA-event pair per step -> per-step milliseconds."""
+    """K steps, L2 flushed before each, one CUDA-event pair per step -> (per-step milliseconds, what the last step
+    returned)."""
     starts = [torch.cuda.Event(enable_timing=True) for _ in range(K)]
     ends = [torch.cuda.Event(enable_timing=True) for _ in range(K)]
     torch.cuda.synchronize()
     for k in range(K):
         flush(k)
         starts[k].record()
-        env.step(pool[k % len(pool)])
+        last = env.step(pool[k % len(pool)])
         ends[k].record()
     torch.cuda.synchronize()
-    return np.array([s.elapsed_time(e) for s, e in zip(starts, ends)], dtype=np.float64)
+    return np.array([s.elapsed_time(e) for s, e in zip(starts, ends)], dtype=np.float64), last
+
+
+def dump_outputs(directory, step_result):
+    """Write one step's (obs, reward, terminated, truncated, infos) as float32 / float64 .npy files in `directory`,
+    at most DUMP_LIMIT_BYTES in all (a seeded sample of env rows beyond that)."""
+    obs, rew, term, trunc, infos = step_result
+    done = (term | trunc).cpu().numpy()
+    final = infos["final_observation"].cpu().numpy().astype(np.float32)
+    final[~done] = 0.0   # only the finished envs' rows are defined
+    arrays = {"obs": obs.cpu().numpy().astype(np.float32), "reward": rew.cpu().numpy().astype(np.float64),
+              "terminated": term.cpu().numpy().astype(np.float32), "truncated": trunc.cpu().numpy().astype(np.float32),
+              "final_observation": final}
+    n = len(done)
+    row_bytes = sum(a.nbytes for a in arrays.values()) // n
+    budget = DUMP_LIMIT_BYTES - 4096   # room for the .npy headers
+    if row_bytes * n > budget:
+        keep = budget // (row_bytes + 8)   # 8: the float64 row index written beside them
+        rows = np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a))
 
 
 def extra_config_line(torch, gym_b200, env_id, log2n, steps, dev, flush, peak):
@@ -343,7 +376,7 @@ def extra_config_line(torch, gym_b200, env_id, log2n, steps, dev, flush, peak):
     warm = 250 if is_box2d(env_id) else 20   # Box2D: reach the steady state of random play (contacts, resets)
     for w in range(warm):
         env.step(pool[w % 8])
-    ms = time_steps_flushed(torch, env, pool, steps, flush)
+    ms, _ = time_steps_flushed(torch, env, pool, steps, flush)
     env.close()
     med = float(np.median(ms))
     bpe = BYTES_PER_ENV_STEP.get(env_id, 0)
@@ -365,7 +398,7 @@ def uint8_actions_line(torch, gym_b200, log2n, steps, dev, flush, peak, e2e_step
     pool = [torch.randint(0, 2, (n,), device=dev, dtype=torch.uint8, generator=gen) for _ in range(8)]
     for w in range(20):
         env.step(pool[w % 8])
-    ms = time_steps_flushed(torch, env, pool, steps, flush)
+    ms, _ = time_steps_flushed(torch, env, pool, steps, flush)
     env.close()
     med = float(np.median(ms))
     bpe = BYTES_PER_ENV_STEP[ENV_ID] - 7
@@ -462,7 +495,9 @@ def run_b200(args):
     # the parked envs, compacted reset kernel -- DESIGN.md 4.4)
     launches_per_step = 3 if is_box2d(args.env) else 1
     if world == 1:
-        per_step = time_steps_flushed(torch, env, pool, K, flush)
+        per_step, last = time_steps_flushed(torch, env, pool, K, flush)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
         ms_median, ms_mean = float(np.median(per_step)), float(per_step.mean())
         ms_per_step = ms_median
         kernel_ms = ms_median

@@ -6,7 +6,7 @@ SURVEY.md 8(d) "CPU path timing": ``gym.vector.SyncVectorEnv`` (a serial Python 
 {4, 1024} and ``gym.vector.AsyncVectorEnv`` (one worker process per env, shared-memory observations) with one env
 per host core, >= `seconds` of wall time each after 3 warm-up steps, random actions from ``action_space.sample()``,
 autoreset on.  Runs in its own process (bench.py spawns it before CUDA is touched: AsyncVectorEnv forks).
-Test / measurement infrastructure: uses ``oracle/_ref`` (or /root/reference), never the engine.
+Test / measurement infrastructure: uses ``oracle/_ref``, never the engine.
 """
 import argparse
 import json

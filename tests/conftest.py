@@ -9,7 +9,9 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
+# what the reference (openai/gym 0.26.2) returned in the comparisons of the *_reference* tests
+# (oracle/gen_reference_golden.py)
+REFERENCE_GOLDEN = os.path.join(GOLDEN, "reference")
 
 
 def pytest_configure(config):
@@ -38,6 +40,11 @@ def oracle_mod():
     from oracle import oracle
     oracle.build()
     return oracle
+
+
+def load_reference_golden(name):
+    z = np.load(os.path.join(REFERENCE_GOLDEN, name + ".npz"))
+    return {k: (str(z[k]) if z[k].dtype.kind == "U" and z[k].ndim == 0 else z[k]) for k in z.files}
 
 
 def have_cuda():

@@ -1,57 +1,36 @@
-"""Oracle (and the host-side space objects) against the LIVE reference.
+"""Oracle (and the host-side space objects) against the reference.
 
-Runs only where /root/reference exists (the build container); on the GPU box
-the committed fixtures in tests/golden stand in for it.
+The first two tests compare with what the reference (openai/gym 0.26.2) returned for the same seeds and actions,
+stored in tests/golden/reference by oracle/gen_reference_golden.py.  The registry test runs gym's own registry, so it
+needs the reference installed in oracle/_ref (oracle/make_ref.py) and skips without it.
 """
-import os
-import sys
-import warnings
-
 import numpy as np
 import pytest
 
-from conftest import REFERENCE
+from conftest import load_reference_golden
+from oracle import ref_gym
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="reference tree not present")
-
-
-@pytest.fixture(scope="module")
-def gym():
-    for n, v in (("bool8", np.bool_), ("float_", np.float64)):
-        if not hasattr(np, n):
-            setattr(np, n, v)
-    sys.path.insert(0, REFERENCE)
-    warnings.filterwarnings("ignore")
-    import gym as ref
-    yield ref
-    sys.path.remove(REFERENCE)
+CLASSIC = ["CartPole-v1", "MountainCar-v0", "MountainCarContinuous-v0", "Pendulum-v1", "Acrobot-v1"]
 
 
-def _actions(env_id, rng, T, N):
-    if env_id.startswith("CartPole"):
-        return rng.integers(0, 2, size=(T, N))
-    if env_id.startswith(("MountainCar-", "Acrobot")):
-        return rng.integers(0, 3, size=(T, N))
-    lim = 2.5 if env_id.startswith("Pendulum") else 1.3
-    return rng.uniform(-lim, lim, size=(T, N, 1)).astype(np.float32)
-
-
-@pytest.mark.parametrize("env_id", ["CartPole-v1", "MountainCar-v0", "MountainCarContinuous-v0",
-                                    "Pendulum-v1", "Acrobot-v1"])
-def test_oracle_bit_exact_against_live_reference(gym, oracle_mod, env_id):
-    N, T, seed = 6, 260, 4242
-    rng = np.random.default_rng(77)
-    acts = _actions(env_id, rng, T, N)
-    envs = gym.vector.SyncVectorEnv([lambda: gym.make(env_id, disable_env_checker=True) for _ in range(N)])
+@pytest.mark.parametrize("env_id", CLASSIC)
+def test_oracle_bit_exact_against_reference_golden(oracle_mod, env_id):
+    """Against the golden roll-out of the reference's SyncVectorEnv: 8 envs, seed 31337, 320 random steps
+    (tests/golden/reference/sync_vector_<id>.npz, also the one the engine is checked against in
+    tests/test_gpu_reference_live.py)."""
+    g = load_reference_golden(f"sync_vector_{env_id}")
+    N, T, seed = 8, 320, 31337
+    acts = g["actions"]
+    assert acts.shape[:2] == (T, N) and int(g["seed"]) == seed
     v = oracle_mod.OracleVec(env_id, N)
-    ref_obs, _ = envs.reset(seed=seed)
+    ref_obs = g["obs0"]
     obs = v.reset(seed=seed)
     if env_id.startswith("Acrobot"):
         np.testing.assert_allclose(obs, ref_obs, rtol=2e-7)
     else:
         assert np.array_equal(obs, ref_obs)
     for t in range(T):
-        ro, rr, rte, rtr, info = envs.step(acts[t])
+        ro, rr, rte, rtr = g["obs"][t], g["reward"][t], g["terminated"][t], g["truncated"][t]
         o, r, te, tr, fo = v.step(acts[t])
         assert np.array_equal(te, rte) and np.array_equal(tr, rtr)
         assert np.array_equal(r, rr)
@@ -61,39 +40,39 @@ def test_oracle_bit_exact_against_live_reference(gym, oracle_mod, env_id):
             assert np.array_equal(o[~done], ro[~done])
         else:
             assert np.array_equal(o, ro)
+        assert np.array_equal(g["final_mask"][t], done)
         for i in np.flatnonzero(done):
-            assert np.array_equal(info["final_observation"][i], fo[i])
-    envs.close()
+            assert np.array_equal(g["final_obs"][t, i], fo[i])
     v.close()
 
 
-def test_space_objects_sample_like_the_reference(gym):
+def test_space_objects_sample_like_the_reference():
+    """Bounds, 5 samples after action_space.seed(5), one batch_space(7) sample after seed(9), per env
+    (tests/golden/reference/spaces.npz)."""
     from gym_b200 import spaces
     from gym_b200.envs import KINDS
-    ref_ids = {0: "CartPole-v1", 1: "MountainCar-v0", 2: "MountainCarContinuous-v0", 3: "Pendulum-v1",
-               4: "Acrobot-v1"}
-    for kind, env_id in ref_ids.items():
-        ref = gym.make(env_id, disable_env_checker=True)
+    g = load_reference_golden("spaces")
+    for kind, env_id in enumerate(CLASSIC):
+        ref = {k.split("__", 1)[1]: v for k, v in g.items() if k.startswith(env_id + "__")}
         obs_space, act_space = KINDS[kind].spaces(None)
-        assert obs_space.shape == ref.observation_space.shape
-        assert np.array_equal(obs_space.low, ref.observation_space.low)
-        assert np.array_equal(obs_space.high, ref.observation_space.high)
-        ref.action_space.seed(5)
+        assert obs_space.shape == tuple(ref["obs_shape"])
+        assert np.array_equal(obs_space.low, ref["obs_low"])
+        assert np.array_equal(obs_space.high, ref["obs_high"])
         act_space.seed(5)
-        for _ in range(5):
-            assert np.array_equal(np.asarray(act_space.sample()), np.asarray(ref.action_space.sample()))
-        rb = gym.vector.utils.batch_space(ref.action_space, 7)
+        for k in range(5):
+            assert np.array_equal(np.asarray(act_space.sample()), ref["samples"][k])
         mb = spaces.batch_space(act_space, 7)
-        rb.seed(9)
         mb.seed(9)
-        assert np.array_equal(mb.sample(), rb.sample())
-        assert type(mb).__name__ == type(rb).__name__ and mb.shape == rb.shape and mb.dtype == rb.dtype
-        ref.close()
+        assert np.array_equal(mb.sample(), ref["batch_sample"])
+        assert (type(mb).__name__ == str(ref["batch_type"]) and mb.shape == tuple(ref["batch_shape"])
+                and str(mb.dtype) == str(ref["batch_dtype"]))
 
 
-def test_plugin_registers_engine_ids_in_the_real_registry(gym):
+@pytest.mark.skipif(ref_gym.reference_path() is None, reason="needs the reference installed in oracle/_ref")
+def test_plugin_registers_engine_ids_in_the_real_registry():
     """gym/envs/registration.py:266-309,434-499: the ids resolve through gym's own registry and gym.make
     reaches the engine's constructor (which refuses to run without a B200: no CPU fallback)."""
+    gym = ref_gym.import_reference()
     import gym_b200
     from gym_b200 import error, plugin
     ids = plugin.register_all()
