@@ -61,37 +61,14 @@ struct b200gym {
         unsigned long long *ring = nullptr, *counter = nullptr; int ring_size = 0;
     } ep;
     int sm_count = 148;
-    int occ[B200GYM_NUM_KINDS][3][4] = {};  // cached CTAs/SM of step_kernel_persistent per (kind, action width, lean + 2 * deep)
-    int p_depth = 1;                        // kernel P/L: tiles in flight per thread (B200GYM_P_DEPTH=1|2)
-    int p_ctas = -1;                        // kernel P/L: resident CTAs per SM; -1 = occupancy limit, 0 = balance the tile
-                                            // rounds (see launch_step_typed), k > 0 = exactly k (B200GYM_P_CTAS, tuning runs)
+    int occ[B200GYM_NUM_KINDS][3][2] = {};  // cached CTAs/SM of step_kernel_persistent per (kind, action width, lean)
     int kernel_choice = 2;                  // 0: kernel A (one tile per CTA), 1: kernel P (resident grid, asynchronous
                                             // prefetch, deferred resets), 2: P's lean instantiation where it applies
                                             // (else P); B200GYM_KERNEL=a|p|l overrides
-    int gather_bulk = 1;                    // multi-GPU step: 1 = kernel G (staged tile + bulk pushes), 0 = per-thread
-                                            // peer stores from kernel A; B200GYM_GATHER=bulk|direct overrides
-    int block_a = 256;                      // CTA size of kernel A (B200GYM_BLOCK_A=64|128|256, tuning runs)
-    int box2d_block = 128;                  // LunarLander step kernel: CTA size (B200GYM_BOX2D_BLOCK=128|256, tuning runs)
-    int box2d_defer = 1;                    // Box2D tasks: 1 = the autoresets of a step run in a last, compacted kernel
-                                            // (B200GYM_BOX2D_DEFER=0: inline).  Neutral in round 1; with the TOI kernel
-                                            // it takes reset() + its embedded world step off the critical path of the
-                                            // envs that crash in a TOI sub-step (LunarLander 1.83 -> 1.74 ms, BipedalWalker
-                                            // 7.9 -> 7.4 ms per 2^16-env step)
-    int box2d_split = 0;                    // Box2D tasks: 1 = the step kernel's resets overlap the TOI kernel on a side stream
-                                            // (B200GYM_BOX2D_SPLIT=1).  Measured neutral (LunarLander 1.81 vs 1.82 ms,
-                                            // BipedalWalker 7.62 vs 7.67): the envs that end an episode are mostly the parked
-                                            // ones, whose resets can only follow the TOI kernel -- so the plain sequence is
-                                            // the default
-    int toi_grid = 12;                      // TOI kernel: one-warp CTAs per SM (B200GYM_TOI_GRID, tuning runs)
-    int box2d_toi_defer = 1;                // Box2D tasks: 1 = envs with a possible TOI event finish in the compacted TOI kernel
-                                            // (B200GYM_BOX2D_TOI_DEFER=0: SolveTOI inline in the step kernel)
+    // Box2D tasks (see launch_box2d_step)
     int32_t *toi_list = nullptr;            // [n] env offsets parked for the TOI kernel, per launch range
     int32_t *toi_count = nullptr;           // [kResetSlots]
     uint32_t *toi_mid = nullptr;            // [kToiMidWords][n] SoA side buffer of the parked envs
-    int32_t *reset_list2 = nullptr;         // [n] / [kResetSlots]: the resets of the TOI kernel (its own list, so that the
-    int32_t *reset_count2 = nullptr;        // step kernel's resets can run on the side stream while the TOI kernel runs)
-    cudaStream_t side = nullptr;            // Box2D tasks: side stream of the step-kernel resets (fork / join by events)
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     int32_t *reset_list = nullptr;          // [n] env offsets to reset, filled per launch range
     int32_t *reset_count = nullptr;         // [kResetSlots] one counter per concurrently running launch range
     // fused all-gather over peer memory (b200gym_p2p_*)
@@ -111,15 +88,6 @@ struct b200gym {
     unsigned long long *h_invalid = nullptr;   // page-locked landing word of the invalid-action counter
     cudaEvent_t hevent = nullptr;
     unsigned long long **d_peer_flags = nullptr;
-    unsigned int *p2p_done = nullptr;       // CTA counter of kernel G's fused step barrier
-    bool p2p_barrier_fused = false;         // set by the last launch_step: the barrier ran in kernel G's tail
-    int p2p_fuse = 0;                       // B200GYM_P2P_FUSE_BARRIER=1: the step barrier in kernel G's tail instead of the
-                                            // 32-thread p2p_sync_kernel.  Correct (tests/test_gpu_multi.py runs it) but
-                                            // measured SLOWER on 2 x B200, 82 vs 59 us per step: to vouch for its pushes a
-                                            // CTA must wait for their COMPLETION (cp.async.bulk.wait_group 0: an NVLink
-                                            // round trip per tile) instead of only for its tile to be read out of shared
-                                            // memory, and that costs more residency than the kernel boundary + one tiny
-                                            // launch save -- so the separate launch stays the default
     cudaStream_t hstream[2] = {nullptr, nullptr};
     bool host_ready = false;
     mutable std::string err;
@@ -190,17 +158,15 @@ struct StepArgs {
     double param0;
     lunar::Opts lunar_opts;   // LunarLander constructor variants (uniform over the batch)
     // Box2D tasks: envs whose episode ended in this launch are appended here (offset from `first`) and reset by
-    // the *_reset_list_kernel that follows on the stream; nullptr: reset inline
+    // box2d_reset_list_kernel, which follows on the stream
     int32_t *reset_list;
     int32_t *reset_count;
     // Box2D tasks: envs whose step may contain a continuous-collision event (b2l::toi_needed) are parked after the
-    // discrete solve -- world record + the sweep starts / env intermediates in toi_mid -- and finished by the
-    // *_toi_kernel that follows on the stream, in warps full of such envs; nullptr: everything inline
+    // discrete solve -- world record + the sweep starts / env intermediates in toi_mid -- and finished by
+    // box2d_toi_kernel, which follows on the stream, in warps full of such envs
     int32_t *toi_list;
     int32_t *toi_count;
     uint32_t *toi_mid;
-    // fused all-gather (multi-GPU): every result is ALSO stored into the same rows of the peers'
-    // gather buffers over NVLink (peer-mapped pointers, slice offset already applied)
     // RecordEpisodeStatistics fused into the step (b200gym_set_episode_stats; nullptr = off): float32 return and
     // int32 length accumulators, infos["episode"]["r"/"l"] rows of finishing envs, ring of recent episodes
     float *ep_acc;
@@ -209,17 +175,10 @@ struct StepArgs {
     int32_t *ep_l;
     unsigned long long *ep_ring, *ep_counter;
     int32_t ep_ring_size;
-    // fused all-gather: the step barrier in kernel G's tail (null = the separate p2p_sync_kernel / no exchange).  The
-    // last CTA of the launch to finish its pushes publishes "my rows of step `p2p_step` are in your buffers" to every
-    // peer and waits for theirs, so the exchange costs no launch of its own
-    unsigned int *p2p_done;                       // device counter of finished CTAs (reset by the last one)
-    unsigned long long *const *p2p_peer_flags;    // [world] -> rank r's flag words (mapped)
-    const unsigned long long *p2p_my_flags;
-    int *p2p_timed_out;
-    unsigned long long p2p_step, p2p_timeout_ns;
-    int32_t p2p_world, p2p_rank;
     int32_t bulk_sink;   // 1: use kernel G's staged bulk stores even without peers (host path: the output arrays are
                          // mapped host memory, where many small stores are what hurts)
+    // fused all-gather (multi-GPU): every result is ALSO stored into the same rows of the peers'
+    // gather buffers over NVLink (peer-mapped pointers, slice offset already applied)
     int32_t npeer;
     float *peer_obs[B200GYM_MAX_PEERS];
     double *peer_reward[B200GYM_MAX_PEERS];
@@ -335,9 +294,6 @@ struct StagedSink {
 //   48 / 5: A 26.7, P 24.6, lean P 24.6.   -> 6 CTAs/SM (40 registers, no spills in the lean loop).
 #ifndef B200_MIN_CTAS
 #define B200_MIN_CTAS 6
-#endif
-#ifndef B200_STAGES
-#define B200_STAGES 2
 #endif
 template <int KIND>
 struct Tuning {
@@ -473,7 +429,6 @@ __device__ __forceinline__ void ld_async(void *smem_dst, const void *gmem_src) {
 }
 __device__ __forceinline__ void ld_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void ld_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void ld_wait_all_but_one() { asm volatile("cp.async.wait_group 1;" ::: "memory"); }
 
 // bulk (TMA, SASS UBLKCP) shared -> global store of a contiguous block; works on peer-mapped addresses
 __device__ __forceinline__ void st_bulk(void *gmem_dst, const void *smem_src, uint32_t bytes) {
@@ -483,8 +438,6 @@ __device__ __forceinline__ void st_bulk(void *gmem_dst, const void *smem_src, ui
 }
 __device__ __forceinline__ void st_bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void st_bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-// ... until the bulk copies of this thread are COMPLETE (their writes performed), not just their source read
-__device__ __forceinline__ void st_bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 // generic-proxy writes to shared memory -> visible to the async proxy that executes the bulk copy
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
@@ -523,16 +476,14 @@ struct PrefetchLayout {
 // LEAN (the single-GPU step without the fused RecordEpisodeStatistics, fewer than 2^31 envs): 32-bit env indices
 // (one IMAD.WIDE per address instead of a 64-bit add chain), no per-peer store loops, no episode accounting --
 // same arithmetic, same stores, fewer issue slots.
-template <int KIND, typename ActT, bool LEAN, int DEPTH>
+template <int KIND, typename ActT, bool LEAN>
 __global__ void __launch_bounds__(kThreads, Tuning<KIND>::kMinCtas) step_kernel_persistent(const StepArgs a, const int num_tiles) {
     using E = Env<KIND>;
     using L = PrefetchLayout<KIND, ActT>;
     using Idx = typename std::conditional<LEAN, uint32_t, int64_t>::type;
-    static_assert(DEPTH == 1 || DEPTH == 2, "one or two tiles in flight per thread");
-    // DEPTH stages of per-thread input slots: the tile being advanced + DEPTH tiles in flight behind it would need
-    // DEPTH + 1 stages if a slot were still in use while its refill is issued; it is not -- a thread moves its slot
-    // into registers before it refills it -- so DEPTH stages hold DEPTH tiles in flight
-    __shared__ __align__(16) unsigned char in_mem[DEPTH * L::kBytes];
+    // one stage of per-thread input slots holds the next tile in flight: a thread moves its slot into registers
+    // before it refills it
+    __shared__ __align__(16) unsigned char in_mem[L::kBytes];
     __shared__ int reset_list[kResetCap];
     __shared__ int reset_count;
     const int tid = threadIdx.x;
@@ -543,8 +494,8 @@ __global__ void __launch_bounds__(kThreads, Tuning<KIND>::kMinCtas) step_kernel_
     const DirectSinkT<!LEAN> sink{a};
     const Idx first = (Idx)a.first, count = (Idx)a.count;
 
-    auto prefetch = [&](int tile, int stage) {
-        unsigned char *base = in_mem + stage * L::kBytes;
+    auto prefetch = [&](int tile) {
+        unsigned char *base = in_mem;
         double *s_state = reinterpret_cast<double *>(base + L::kStateOff);
         int32_t *s_elapsed = reinterpret_cast<int32_t *>(base + L::kElapsedOff);
         const Idx j = (Idx)tile * kThreads + tid;
@@ -560,26 +511,23 @@ __global__ void __launch_bounds__(kThreads, Tuning<KIND>::kMinCtas) step_kernel_
     };
 
     int tile = blockIdx.x;
-    prefetch(tile, 0);
-    if constexpr (DEPTH == 2) prefetch(tile + (int)gridDim.x, 1);
-    int stage = 0;
+    prefetch(tile);
     for (; tile < num_tiles; tile += gridDim.x) {
         const Idx j = (Idx)tile * kThreads + tid;
         const bool in_range = j < count;
         const Idx i = first + j;
         ActT av{};
         if constexpr (!L::kActAsync) { if (in_range) av = __ldg(actions + (size_t)i * L::kActPerEnv); }
-        if constexpr (DEPTH == 2) acp::ld_wait_all_but_one(); else acp::ld_wait_all();
-        unsigned char *base = in_mem + stage * L::kBytes;
+        acp::ld_wait_all();
+        unsigned char *base = in_mem;
         const double *s_state = reinterpret_cast<const double *>(base + L::kStateOff);
         double s[E::S];
 #pragma unroll
         for (int k = 0; k < E::S; k++) s[k] = s_state[k * kThreads + tid];
         const int32_t elapsed = reinterpret_cast<const int32_t *>(base + L::kElapsedOff)[tid];
         if constexpr (L::kActAsync) av = *reinterpret_cast<const ActT *>(base + L::kActOff + tid * L::kActBytes);
-        // this thread's slots are in registers now: refill them with its env DEPTH tiles ahead
-        prefetch(tile + DEPTH * (int)gridDim.x, stage);
-        if constexpr (DEPTH == 2) stage ^= 1;
+        // this thread's slots are in registers now: refill them with its env in the next tile
+        prefetch(tile + (int)gridDim.x);
         long long action_int = 0;
         float a0 = 0.0f;
         if constexpr (E::A == 0) action_int = (long long)av;
@@ -654,36 +602,7 @@ __global__ void __launch_bounds__(kThreads, Tuning<KIND>::kMinCtas) step_kernel_
         acp::st_bulk(term + i0, s_term, kThreads);
         acp::st_bulk(trunc + i0, s_trunc, kThreads);
         acp::st_bulk_commit();
-        if (a.p2p_done) acp::st_bulk_wait_all();   // the step barrier below vouches for these writes
-        else acp::st_bulk_wait_read();             // the tile must stay in shared memory until the copy engine has read it
-    }
-    if (a.p2p_done) {
-        // the exchange's step barrier, fused: every CTA counts itself in once its pushes are complete; the last one
-        // of this rank tells every peer "my rows of this step are in your buffers" and waits for theirs
-        __syncthreads();
-        __shared__ int is_last;
-        if (threadIdx.x == 0) {
-            __threadfence_system();
-            const unsigned prev = atomicAdd(a.p2p_done, 1u);
-            is_last = prev == gridDim.x - 1;
-            if (is_last) *a.p2p_done = 0u;         // for the next launch (this one has no more increments coming)
-        }
-        __syncthreads();
-        if (is_last && (int)threadIdx.x < a.p2p_world && (int)threadIdx.x != a.p2p_rank) {
-            const int p = threadIdx.x;
-            __threadfence_system();
-            volatile unsigned long long *f = a.p2p_peer_flags[p] + a.p2p_rank;
-            *f = a.p2p_step;
-            const volatile unsigned long long *w = a.p2p_my_flags + p;
-            const unsigned long long t0 = global_ns();
-            while (*w < a.p2p_step) {
-                if (global_ns() - t0 > a.p2p_timeout_ns) {
-                    atomicExch(a.p2p_timed_out, p + 1);
-                    break;
-                }
-            }
-            __threadfence_system();
-        }
+        acp::st_bulk_wait_read();   // the tile must stay in shared memory until the copy engine has read it
     }
 }
 
@@ -743,13 +662,20 @@ __global__ void __launch_bounds__(kThreads) state_set_kernel(double *soa, const 
     for (int k = 0; k < S; k++) soa[k * n + i] = aos[i * S + k];
 }
 
-// ---- LunarLander-v2 (lunar.cuh): one thread per env, the whole b2World::Step in registers/local ----
-constexpr int kLunarThreads = 128;
+// ---- the Box2D tasks (lunar.cuh, walker.cuh): one thread per env, the whole b2World::Step in registers/local ----
+// A step is three launches on the stream:
+//   box2d_step_kernel        validates the action and runs env_pre without SolveTOI; an env whose step may contain a
+//                            continuous-collision event is parked (record + toi_mid) for the TOI kernel, every other
+//                            env finishes here
+//   box2d_toi_kernel         b2l::solve_toi of the parked envs, in warps full of them, then finish
+//   box2d_reset_list_kernel  the autoresets of the step, compacted
+// Finish (box2d_finish) is env_post, TimeLimit, the outputs and the episode statistics; an env whose episode ended
+// goes onto the reset list.  What differs between the tasks -- record, what crosses the park, env_pre / env_post, the
+// per-env reset, register budgets -- is in the task types below (LunarTask, LunarStep, WalkerTask).
+constexpr int kBox2dThreads = 128;
 constexpr int kResetSlots = 64;   // launch ranges of one handle that may be in flight at once (host path: <= 64 chunks)
 
-constexpr int kLunarMaxThreads = 256;
-
-// The TOI kernels run one warp per CTA and give each warp as FEW parked envs as the resident grid allows: the lanes
+// The TOI kernel runs one warp per CTA and gives each warp as FEW parked envs as the resident grid allows: the lanes
 // of a warp diverge completely in this code (different contact lists, GJK / root-finder trip counts, event counts),
 // so a warp takes the SUM of its lanes' paths, and with a few thousand parked envs on 148 SMs there are more warp
 // slots than envs.  Measured (LunarLander, 2^16 envs, ~3 300 parked per step, ncu): 32 envs per warp 1.19 ms for
@@ -759,115 +685,202 @@ __device__ __forceinline__ int toi_lanes_per_warp(int cnt, int nwarps) {
     const int L = (cnt + nwarps - 1) / nwarps;
     return L < 1 ? 1 : (L > 32 ? 32 : L);
 }
+// One-warp CTAs per SM of the TOI kernel; the kernel strides over the list.  12 warps of up to 168 registers per thread
+// fit in an SM's 65 536 registers at once (12 x 32 x 168 = 64 512), which covers every TOI instantiation.  Larger grids
+// (fewer envs per warp) were measured: LunarLander 1.74 / 1.82 / 1.85 ms at 12 / 64 / 256 CTAs per SM, BipedalWalker
+// (nearly every env parked) 7.4 / 12.2 / 17.1 ms
+constexpr int kToiCtasPerSm = 12;
 
-// side buffer of a parked env ([kToiMidWords][n] SoA): the sweep starts of the 3 bodies + env_pre's intermediates
+// side buffer of a parked env ([kToiMidWords][n] SoA): the sweep starts of the bodies + env_pre's intermediates
 constexpr int kToiMidWords = 20;   // LunarLander uses 13, BipedalWalker 15
 
-__device__ __forceinline__ void lunar_store_mid(const StepArgs &a, int64_t i, const lunar::World &W, const lunar::Mid &mid) {
+__device__ __forceinline__ void store_sweep_starts(const StepArgs &a, int64_t i, const b2l::Body *b, int nb) {
     uint32_t *m = a.toi_mid + i;
-    for (int b = 0; b < lunar::NB; b++) {
-        m[(int64_t)(3 * b + 0) * a.n] = __float_as_uint(W.b[b].c0.x);
-        m[(int64_t)(3 * b + 1) * a.n] = __float_as_uint(W.b[b].c0.y);
-        m[(int64_t)(3 * b + 2) * a.n] = __float_as_uint(W.b[b].a0);
+    for (int k = 0; k < nb; k++) {
+        m[(int64_t)(3 * k + 0) * a.n] = __float_as_uint(b[k].c0.x);
+        m[(int64_t)(3 * k + 1) * a.n] = __float_as_uint(b[k].c0.y);
+        m[(int64_t)(3 * k + 2) * a.n] = __float_as_uint(b[k].a0);
     }
-    const unsigned long long mc = (unsigned long long)__double_as_longlong(mid.main_cost);
-    const unsigned long long sc = (unsigned long long)__double_as_longlong(mid.side_cost);
-    m[(int64_t)9 * a.n] = (uint32_t)mc; m[(int64_t)10 * a.n] = (uint32_t)(mc >> 32);
-    m[(int64_t)11 * a.n] = (uint32_t)sc; m[(int64_t)12 * a.n] = (uint32_t)(sc >> 32);
 }
-
-__device__ __forceinline__ void lunar_load_mid(const StepArgs &a, int64_t i, lunar::World &W, lunar::Mid &mid) {
+__device__ __forceinline__ void load_sweep_starts(const StepArgs &a, int64_t i, b2l::Body *b, int nb) {
     const uint32_t *m = a.toi_mid + i;
-    for (int b = 0; b < lunar::NB; b++) {
-        W.b[b].c0.x = __uint_as_float(m[(int64_t)(3 * b + 0) * a.n]);
-        W.b[b].c0.y = __uint_as_float(m[(int64_t)(3 * b + 1) * a.n]);
-        W.b[b].a0 = __uint_as_float(m[(int64_t)(3 * b + 2) * a.n]);
+    for (int k = 0; k < nb; k++) {
+        b[k].c0.x = __uint_as_float(m[(int64_t)(3 * k + 0) * a.n]);
+        b[k].c0.y = __uint_as_float(m[(int64_t)(3 * k + 1) * a.n]);
+        b[k].a0 = __uint_as_float(m[(int64_t)(3 * k + 2) * a.n]);
     }
-    mid.main_cost = __longlong_as_double((long long)(((unsigned long long)m[(int64_t)10 * a.n] << 32) | m[(int64_t)9 * a.n]));
-    mid.side_cost = __longlong_as_double((long long)(((unsigned long long)m[(int64_t)12 * a.n] << 32) | m[(int64_t)11 * a.n]));
-    mid.awake = true;   // only awake islands are parked
 }
 
-// everything after world.Step of LunarLander.step, then TimeLimit, outputs and the same-step autoreset
-__device__ __noinline__ void lunar_finish(const StepArgs &a, int64_t i, int64_t j, lunar::World &W, Pcg64 &g, int32_t elapsed,
-                                          const lunar::Mid &mid) {
-    const lunar::Opts &O = a.lunar_opts;
-    float obs[8];
+// LunarLander.  The phases after the step kernel do not read the action, so all four step instantiations (LunarStep)
+// share this type's TOI and reset-list kernels.
+struct LunarTask {
+    using World = lunar::World;
+    using Scene = lunar::Scene;
+    struct Carry { Pcg64 g; lunar::Mid mid; };   // the env's PCG64 stream, env_pre's intermediates
+    static constexpr int kObs = 8;
+    static constexpr int kResetMinBlocks = 0;    // __launch_bounds__ of the reset-list kernel: no minimum
+    static __device__ __forceinline__ void load(const StepArgs &a, int64_t i, World &W, Carry &c) {
+        lunar::load_world(W, a.lunar_rec, a.n, i, a.lunar_opts.wind != 0);
+        c.g = pcg64_load(a.rng + 4 * i);
+    }
+    static __device__ __forceinline__ void store(const StepArgs &a, int64_t i, const World &W, const Carry &c) {
+        lunar::store_world(W, a.lunar_rec, a.n, i, a.lunar_opts.wind != 0);
+        pcg64_store(a.rng + 4 * i, c.g);
+    }
+    static __device__ __forceinline__ void store_mid(const StepArgs &a, int64_t i, const World &W, const Carry &c) {
+        store_sweep_starts(a, i, W.b, lunar::NB);
+        uint32_t *m = a.toi_mid + i;
+        const unsigned long long mc = (unsigned long long)__double_as_longlong(c.mid.main_cost);
+        const unsigned long long sc = (unsigned long long)__double_as_longlong(c.mid.side_cost);
+        m[(int64_t)9 * a.n] = (uint32_t)mc; m[(int64_t)10 * a.n] = (uint32_t)(mc >> 32);
+        m[(int64_t)11 * a.n] = (uint32_t)sc; m[(int64_t)12 * a.n] = (uint32_t)(sc >> 32);
+    }
+    static __device__ __forceinline__ void load_mid(const StepArgs &a, int64_t i, World &W, Carry &c) {
+        load_sweep_starts(a, i, W.b, lunar::NB);
+        const uint32_t *m = a.toi_mid + i;
+        c.mid.main_cost = __longlong_as_double((long long)(((unsigned long long)m[(int64_t)10 * a.n] << 32) | m[(int64_t)9 * a.n]));
+        c.mid.side_cost = __longlong_as_double((long long)(((unsigned long long)m[(int64_t)12 * a.n] << 32) | m[(int64_t)11 * a.n]));
+        c.mid.awake = true;   // only awake islands are parked
+    }
+    static __device__ __forceinline__ void post(World &W, const Carry &c, float (&obs)[kObs], double &reward, bool &terminated) {
+        lunar::env_post(W, c.mid, obs, reward, terminated);
+    }
+    static __device__ __forceinline__ void reset(uint32_t *rec, const int64_t &n, int64_t i, uint64_t *rng, const lunar::Opts &O,
+                                                 float (&obs)[kObs]) {
+        lunar::reset_from_record(rec, n, i, rng, O, obs);
+    }
+};
+
+// the LunarLander step kernel's part: the action encoding (Discrete(4) as ActT, or Box(2) float32 with CONT)
+template <typename ActT, bool CONT>
+struct LunarStep : LunarTask {
+    using Task = LunarTask;
+    // __launch_bounds__(256, 2) although it launches 128-thread CTAs: the register budget of DESIGN §4.4
+    static constexpr int kStepMaxThreads = 256, kStepMinBlocks = 2;
+    struct Action { long long act; float ca0, ca1; };
+    static __device__ __forceinline__ bool read_action(const StepArgs &a, int64_t i, Action &v) {
+        v.act = 0; v.ca0 = 0.0f; v.ca1 = 0.0f;
+        if constexpr (CONT) {
+            const float2 c = __ldg(reinterpret_cast<const float2 *>(a.actions) + i);   // Box(2) float32, lunar_lander.py:285-287
+            v.ca0 = c.x; v.ca1 = c.y;
+            return true;
+        } else {
+            v.act = (long long)__ldg(reinterpret_cast<const ActT *>(a.actions) + i);
+            return !(v.act < 0 || v.act > 3);   // lunar_lander.py:482-484
+        }
+    }
+    // env_pre without SolveTOI; true: the env needs the TOI phase
+    static __device__ __forceinline__ bool pre(const StepArgs &a, World &W, Carry &c, const Action &v) {
+        lunar::env_pre(W, c.g, a.lunar_opts, (int)v.act, v.ca0, v.ca1, lunar::V(0.0f, 0.0f), c.mid, 0u, /*run_toi=*/false);
+        return c.mid.awake && b2l::toi_needed<Scene>(W);
+    }
+};
+
+// BipedalWalker (HC: hardcore).  Step kernel and later phases alike.
+template <bool HC>
+struct WalkerTask {
+    using Task = WalkerTask;
+    using World = walker::World;
+    using Scene = walker::SceneT<HC>;
+    // numpy's 32-bit cache (the record holds it; the PCG64 stream is only drawn by reset()), the action, which
+    // env_post charges for
+    struct Carry { walker::Rng rng; float action[4]; };
+    struct Action { float v[4]; };
+    static constexpr int kObs = 24;
+    static constexpr int kStepMaxThreads = kBox2dThreads, kStepMinBlocks = 4, kResetMinBlocks = 4;
+    static __device__ __forceinline__ void load(const StepArgs &a, int64_t i, World &W, Carry &c) {
+        walker::load_world(W, a.lunar_rec, a.n, i, c.rng, HC);
+    }
+    static __device__ __forceinline__ void store(const StepArgs &a, int64_t i, const World &W, const Carry &c) {
+        walker::store_world(W, a.lunar_rec, a.n, i, c.rng, HC);
+    }
+    static __device__ __forceinline__ void store_mid(const StepArgs &a, int64_t i, const World &W, const Carry &) {
+        store_sweep_starts(a, i, W.b, walker::NB);
+    }
+    // the sweep starts, the action (read again), and the window of obstacle boxes env_pre computed around the hull's
+    // position before the step
+    static __device__ __forceinline__ void load_mid(const StepArgs &a, int64_t i, World &W, Carry &c) {
+        const float4 av = __ldg(reinterpret_cast<const float4 *>(a.actions) + i);
+        c.action[0] = av.x; c.action[1] = av.y; c.action[2] = av.z; c.action[3] = av.w;
+        load_sweep_starts(a, i, W.b, walker::NB);
+        if constexpr (HC) walker::poly_window(W, W.b[0].c0.x - 4.0f, W.b[0].c0.x + 4.0f, W.p_lo, W.p_hi);
+    }
+    static __device__ __forceinline__ bool read_action(const StepArgs &a, int64_t i, Action &v) {
+        const float4 av = __ldg(reinterpret_cast<const float4 *>(a.actions) + i);
+        v.v[0] = av.x; v.v[1] = av.y; v.v[2] = av.z; v.v[3] = av.w;
+        return true;
+    }
+    static __device__ __forceinline__ bool pre(const StepArgs &, World &W, Carry &c, const Action &v) {
+        for (int k = 0; k < 4; k++) c.action[k] = v.v[k];
+        bool awake;
+        walker::env_pre<HC>(W, c.action, walker::V(0.0f, 0.0f), awake, 0u, /*run_toi=*/false);
+        return awake && b2l::toi_needed<Scene>(W);
+    }
+    static __device__ __forceinline__ void post(World &W, const Carry &c, float (&obs)[kObs], double &reward, bool &terminated) {
+        walker::env_post<HC>(W, c.action, false, obs, reward, terminated);
+    }
+    static __device__ __forceinline__ void reset(uint32_t *rec, const int64_t &n, int64_t i, uint64_t *rng, const lunar::Opts &,
+                                                 float (&obs)[kObs]) {
+        walker::reset_from_record<HC>(rec, n, i, rng, obs);
+    }
+};
+
+// everything after world.Step of the task's step(), then TimeLimit, outputs and the same-step autoreset's bookkeeping:
+// the new episode is drawn by box2d_reset_list_kernel, in warps full of resetting envs
+template <typename Task>
+__device__ __noinline__ void box2d_finish(const StepArgs &a, int64_t i, int64_t j, typename Task::World &W,
+                                          const typename Task::Carry &c, int32_t elapsed) {
+    float obs[Task::kObs];
     double reward;
     bool terminated;
-    lunar::env_post(W, mid, obs, reward, terminated);
+    Task::post(W, c, obs, reward, terminated);
     elapsed += 1;                                                        // time_limit.py:51
     const bool truncated = (a.max_steps > 0) && (elapsed >= a.max_steps);
     store_scalars_all(a, i, reward, terminated ? 1 : 0, truncated ? 1 : 0);
     episode_account(a, i, reward, terminated || truncated);
-    bool deferred = false;
-    if ((terminated || truncated) && a.autoreset) {                      // sync_vector_env.py:152-156
-        if (a.final_obs) store_row<8>(a.final_obs, i, obs);
-        if (a.reset_list) {  // the new episode is drawn by lunar_reset_list_kernel, in warps full of resetting envs
-            a.reset_list[a.first + atomicAdd(a.reset_count, 1)] = (int32_t)j;
-            deferred = true;
-        } else {
-            lunar::env_reset(W, g, O, obs);
-            elapsed = 0;
-        }
+    const bool reset = (terminated || truncated) && a.autoreset;        // sync_vector_env.py:152-156
+    if (reset) {
+        if (a.final_obs) store_row<Task::kObs>(a.final_obs, i, obs);
+        a.reset_list[a.first + atomicAdd(a.reset_count, 1)] = (int32_t)j;
     }
-    lunar::store_world(W, a.lunar_rec, a.n, i, O.wind != 0);
-    pcg64_store(a.rng + 4 * i, g);
+    Task::store(a, i, W, c);
     a.elapsed[i] = elapsed;
-    if (!deferred) store_obs_all<8>(a, i, obs);
+    if (!reset) store_obs_all<Task::kObs>(a, i, obs);
 }
 
-template <typename ActT, bool CONT>
-__global__ void __launch_bounds__(kLunarMaxThreads, 2) lunar_step_kernel(const StepArgs a) {
+template <typename Step>
+__global__ void __launch_bounds__(Step::kStepMaxThreads, Step::kStepMinBlocks) box2d_step_kernel(const StepArgs a) {
+    using Task = typename Step::Task;
     const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool in_range = j < a.count;
+    if (j >= a.count) return;
     const int64_t i = a.first + j;
-    long long act = 0;
-    float ca0 = 0.0f, ca1 = 0.0f;
-    bool valid = in_range;
-    if (in_range) {
-        if constexpr (CONT) {
-            const float2 c = __ldg(reinterpret_cast<const float2 *>(a.actions) + i);   // Box(2) float32, lunar_lander.py:285-287
-            ca0 = c.x; ca1 = c.y;
-        } else {
-            act = (long long)__ldg(reinterpret_cast<const ActT *>(a.actions) + i);
-            valid = !(act < 0 || act > 3);   // lunar_lander.py:482-484
-        }
-    }
-    if (!in_range) return;
-    if (!valid) {
+    typename Step::Action act;
+    if (!Step::read_action(a, i, act)) {
         atomicAdd(a.invalid, 1ULL);
         *reinterpret_cast<volatile unsigned long long *>(a.invalid_seen) = 1ULL;
         store_scalars_all(a, i, __longlong_as_double(0x7ff8000000000000LL), 0, 0);
         return;
     }
-    const lunar::Opts &O = a.lunar_opts;
-    lunar::World W;
-    lunar::load_world(W, a.lunar_rec, a.n, i, O.wind != 0);
-    Pcg64 g = pcg64_load(a.rng + 4 * i);
+    typename Task::World W;
+    typename Task::Carry c;
+    Task::load(a, i, W, c);
     const int32_t elapsed = a.elapsed[i];
-    lunar::Mid mid;
-    lunar::env_pre(W, g, O, (int)act, ca0, ca1, lunar::V(0.0f, 0.0f), mid, 0u, /*run_toi=*/false);
-    if (mid.awake && b2l::toi_needed<lunar::Scene>(W)) {
-        if (a.toi_list) {   // park the env for lunar_toi_kernel
-            lunar::store_world(W, a.lunar_rec, a.n, i, O.wind != 0);
-            pcg64_store(a.rng + 4 * i, g);
-            lunar_store_mid(a, i, W, mid);
-            a.toi_list[a.first + atomicAdd(a.toi_count, 1)] = (int32_t)j;
-            return;
-        }
-        b2l::solve_toi<lunar::Scene>(W, (float)(1.0 / 50), true, 0u);
+    if (Step::pre(a, W, c, act)) {   // park the env for box2d_toi_kernel
+        Task::store(a, i, W, c);
+        Task::store_mid(a, i, W, c);
+        a.toi_list[a.first + atomicAdd(a.toi_count, 1)] = (int32_t)j;
+        return;
     }
-    lunar_finish(a, i, j, W, g, elapsed, mid);
+    box2d_finish<Task>(a, i, j, W, c, elapsed);
 }
 
-// The continuous-collision phase of the envs that lunar_step_kernel parked, one warp of parked envs per CTA: the
+// The continuous-collision phase of the envs that box2d_step_kernel parked, one warp of parked envs per CTA: the
 // TOI code (GJK, root finder, the sub-step solver) is large and runs for a few percent of the envs, so it gets
 // its own launch -- dense warps and a warm instruction cache instead of one or two lanes per warp walking it at the
 // end of every warp's critical path -- and the warp-synchronous event rounds of b2l::solve_toi.
-__global__ void __launch_bounds__(32) lunar_toi_kernel(const StepArgs a) {
+template <typename Task>
+__global__ void __launch_bounds__(32) box2d_toi_kernel(const StepArgs a) {
     const int cnt = *a.toi_count;
-    const lunar::Opts &O = a.lunar_opts;
     const int L = toi_lanes_per_warp(cnt, (int)gridDim.x);
     for (int base = blockIdx.x * L; base < cnt; base += gridDim.x * L) {
         const int idx = base + (int)threadIdx.x;
@@ -876,59 +889,46 @@ __global__ void __launch_bounds__(32) lunar_toi_kernel(const StepArgs a) {
         if (on) {
             const int64_t j = a.toi_list[a.first + idx];
             const int64_t i = a.first + j;
-            lunar::World W;
-            lunar::load_world(W, a.lunar_rec, a.n, i, O.wind != 0);
-            lunar::Mid mid;
-            lunar_load_mid(a, i, W, mid);
-            Pcg64 g = pcg64_load(a.rng + 4 * i);
+            typename Task::World W;
+            typename Task::Carry c;
+            Task::load(a, i, W, c);
+            Task::load_mid(a, i, W, c);
             const int32_t elapsed = a.elapsed[i];
-            b2l::solve_toi<lunar::Scene>(W, (float)(1.0 / 50), true, live);
-            lunar_finish(a, i, j, W, g, elapsed, mid);
+            b2l::solve_toi<typename Task::Scene>(W, (float)(1.0 / 50), true, live);
+            box2d_finish<Task>(a, i, j, W, c, elapsed);
         }
     }
 }
 
 // The autoresets of one step, compacted: a lone finishing env would otherwise keep its whole warp waiting through
-// a full reset() (terrain draw + the embedded world step) with one active lane.  Same per-env arithmetic and RNG
-// stream as the inline path.
-__global__ void __launch_bounds__(kLunarThreads) lunar_reset_list_kernel(const StepArgs a) {
+// a full reset() (terrain draw + the embedded world step) with one active lane.
+template <typename Task>
+__global__ void __launch_bounds__(kBox2dThreads, Task::kResetMinBlocks) box2d_reset_list_kernel(const StepArgs a) {
     const int cnt = *a.reset_count;
-    const lunar::Opts &O = a.lunar_opts;
     for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < cnt; idx += gridDim.x * blockDim.x) {
         const int64_t i = a.first + a.reset_list[a.first + idx];
-        lunar::World W;
-        W.flags = a.lunar_rec[(int64_t)lunar::W_FLAGS * a.n + i] & b2l::kFlagsKept;
-        W.wind_idx = O.wind ? (int32_t)a.lunar_rec[(int64_t)lunar::W_WIND * a.n + i] : 0;
-        W.torque_idx = O.wind ? (int32_t)a.lunar_rec[(int64_t)(lunar::W_WIND + 1) * a.n + i] : 0;
-        Pcg64 g = pcg64_load(a.rng + 4 * i);
-        float obs[8];
-        lunar::env_reset(W, g, O, obs);
-        lunar::store_world(W, a.lunar_rec, a.n, i, O.wind != 0);
-        pcg64_store(a.rng + 4 * i, g);
+        float obs[Task::kObs];
+        Task::reset(a.lunar_rec, a.n, i, a.rng, a.lunar_opts, obs);
         a.elapsed[i] = 0;
-        store_obs_all<8>(a, i, obs);
+        store_obs_all<Task::kObs>(a, i, obs);
     }
 }
 
-__global__ void __launch_bounds__(kLunarThreads) lunar_reset_kernel(uint32_t *rec, int32_t *elapsed, uint64_t *rng,
+// reset() of the (masked) envs
+template <typename Task>
+__global__ void __launch_bounds__(kBox2dThreads) box2d_reset_kernel(uint32_t *rec, int32_t *elapsed, uint64_t *rng,
                                                                     const uint8_t *mask, float *obs, int64_t n,
                                                                     const lunar::Opts O) {
-    const int64_t i = (int64_t)blockIdx.x * kLunarThreads + threadIdx.x;
+    const int64_t i = (int64_t)blockIdx.x * kBox2dThreads + threadIdx.x;
     if (i >= n) return;
     if (mask && !mask[i]) return;
-    lunar::World W;
-    W.flags = rec[(int64_t)lunar::W_FLAGS * n + i] & b2l::kFlagsKept;  // the b2World object survives reset()
-    W.wind_idx = O.wind ? (int32_t)rec[(int64_t)lunar::W_WIND * n + i] : 0;          // so do wind_idx / torque_idx
-    W.torque_idx = O.wind ? (int32_t)rec[(int64_t)(lunar::W_WIND + 1) * n + i] : 0;
-    Pcg64 g = pcg64_load(rng + 4 * i);
-    float o[8];
-    lunar::env_reset(W, g, O, o);
-    lunar::store_world(W, rec, n, i, O.wind != 0);
-    pcg64_store(rng + 4 * i, g);
+    float o[Task::kObs];
+    Task::reset(rec, n, i, rng, O, o);
     elapsed[i] = 0;
-    if (obs) store_row<8>(obs, i, o);
+    if (obs) store_row<Task::kObs>(obs, i, o);
 }
 
+// ---- LunarLander-v2 only ------------------------------------------------------------------------------------
 // wind_idx / torque_idx of every env (lunar_lander.py:234-235): two int32 SoA rows of the record
 __global__ void lunar_wind_idx_kernel(uint32_t *rec, int32_t *wind, int32_t *torque, int64_t n, int set) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -963,143 +963,7 @@ static int lunar_upload_consts(b200gym *h) {
     return 0;
 }
 
-// ---- BipedalWalker-v3 (walker.cuh): one thread per env --------------------------------------------
-// everything after world.Step of BipedalWalker.step, then TimeLimit, outputs and the same-step autoreset
-template <bool HC>
-__device__ __noinline__ void walker_finish(const StepArgs &a, int64_t i, int64_t j, walker::World &W, walker::Rng &rng,
-                                           int32_t elapsed, const float (&action)[4]) {
-    float obs[24];
-    double reward;
-    bool terminated;
-    walker::env_post<HC>(W, action, false, obs, reward, terminated);
-    elapsed += 1;                                                        // time_limit.py:51
-    const bool truncated = (a.max_steps > 0) && (elapsed >= a.max_steps);
-    store_scalars_all(a, i, reward, terminated ? 1 : 0, truncated ? 1 : 0);
-    episode_account(a, i, reward, terminated || truncated);
-    bool deferred = false;
-    if ((terminated || truncated) && a.autoreset) {                      // sync_vector_env.py:152-156
-        if (a.final_obs) store_row<24>(a.final_obs, i, obs);
-        if (a.reset_list) {  // drawn by walker_reset_list_kernel (see lunar_reset_list_kernel)
-            a.reset_list[a.first + atomicAdd(a.reset_count, 1)] = (int32_t)j;
-            deferred = true;
-        } else {
-            rng.g = pcg64_load(a.rng + 4 * i);
-            walker::env_reset<HC>(W, rng, obs);
-            pcg64_store(a.rng + 4 * i, rng.g);
-            elapsed = 0;
-        }
-    }
-    walker::store_world(W, a.lunar_rec, a.n, i, rng, HC);
-    a.elapsed[i] = elapsed;
-    if (!deferred) store_obs_all<24>(a, i, obs);
-}
-
-template <bool HC>
-__global__ void __launch_bounds__(kLunarThreads, 4) walker_step_kernel(const StepArgs a) {
-    const int64_t j = (int64_t)blockIdx.x * kLunarThreads + threadIdx.x;
-    if (j >= a.count) return;
-    const int64_t i = a.first + j;
-    const float4 av = __ldg(reinterpret_cast<const float4 *>(a.actions) + i);
-    const float action[4] = {av.x, av.y, av.z, av.w};
-    walker::World W;
-    walker::Rng rng;
-    walker::load_world(W, a.lunar_rec, a.n, i, rng, HC);
-    const int32_t elapsed = a.elapsed[i];
-    bool awake;
-    walker::env_pre<HC>(W, action, walker::V(0.0f, 0.0f), awake, 0u, /*run_toi=*/false);
-    if (awake && b2l::toi_needed<walker::SceneT<HC>>(W)) {
-        if (a.toi_list) {   // park the env for walker_toi_kernel: the record after the discrete solve + the sweep starts
-            walker::store_world(W, a.lunar_rec, a.n, i, rng, HC);
-            uint32_t *m = a.toi_mid + i;
-            for (int b = 0; b < walker::NB; b++) {
-                m[(int64_t)(3 * b + 0) * a.n] = __float_as_uint(W.b[b].c0.x);
-                m[(int64_t)(3 * b + 1) * a.n] = __float_as_uint(W.b[b].c0.y);
-                m[(int64_t)(3 * b + 2) * a.n] = __float_as_uint(W.b[b].a0);
-            }
-            a.toi_list[a.first + atomicAdd(a.toi_count, 1)] = (int32_t)j;
-            return;
-        }
-        b2l::solve_toi<walker::SceneT<HC>>(W, (float)(1.0 / 50), true, 0u);
-    }
-    walker_finish<HC>(a, i, j, W, rng, elapsed, action);
-}
-
-// the continuous-collision phase of the parked envs (see lunar_toi_kernel)
-template <bool HC>
-__global__ void __launch_bounds__(32) walker_toi_kernel(const StepArgs a) {
-    const int cnt = *a.toi_count;
-    const int L = toi_lanes_per_warp(cnt, (int)gridDim.x);
-    for (int base = blockIdx.x * L; base < cnt; base += gridDim.x * L) {
-        const int idx = base + (int)threadIdx.x;
-        const bool on = (int)threadIdx.x < L && idx < cnt;
-        const unsigned live = __ballot_sync(0xffffffffu, on);
-        if (on) {
-            const int64_t j = a.toi_list[a.first + idx];
-            const int64_t i = a.first + j;
-            const float4 av = __ldg(reinterpret_cast<const float4 *>(a.actions) + i);
-            const float action[4] = {av.x, av.y, av.z, av.w};
-            walker::World W;
-            walker::Rng rng;
-            walker::load_world(W, a.lunar_rec, a.n, i, rng, HC);
-            const uint32_t *m = a.toi_mid + i;
-            for (int b = 0; b < walker::NB; b++) {
-                W.b[b].c0.x = __uint_as_float(m[(int64_t)(3 * b + 0) * a.n]);
-                W.b[b].c0.y = __uint_as_float(m[(int64_t)(3 * b + 1) * a.n]);
-                W.b[b].a0 = __uint_as_float(m[(int64_t)(3 * b + 2) * a.n]);
-            }
-            // the window of obstacle boxes env_pre computed around the hull's position before the step
-            if constexpr (HC) walker::poly_window(W, W.b[0].c0.x - 4.0f, W.b[0].c0.x + 4.0f, W.p_lo, W.p_hi);
-            const int32_t elapsed = a.elapsed[i];
-            b2l::solve_toi<walker::SceneT<HC>>(W, (float)(1.0 / 50), true, live);
-            walker_finish<HC>(a, i, j, W, rng, elapsed, action);
-        }
-    }
-}
-
-template <bool HC>
-__global__ void __launch_bounds__(kLunarThreads, 4) walker_reset_list_kernel(const StepArgs a) {
-    const int cnt = *a.reset_count;
-    for (int idx = blockIdx.x * blockDim.x + threadIdx.x; idx < cnt; idx += gridDim.x * blockDim.x) {
-        const int64_t i = a.first + a.reset_list[a.first + idx];
-        walker::World W;
-        walker::Rng r;
-        walker::bind_world(W, a.lunar_rec, a.n, i);
-        W.flags = a.lunar_rec[(int64_t)walker::W_FLAGS * a.n + i] & b2l::kFlagsKept;
-        r.has32 = a.lunar_rec[(int64_t)walker::W_RNG32 * a.n + i];
-        r.val32 = a.lunar_rec[(int64_t)(walker::W_RNG32 + 1) * a.n + i];
-        r.g = pcg64_load(a.rng + 4 * i);
-        W.np = 0; W.p_lo = 0; W.p_hi = -1;
-        float obs[24];
-        walker::env_reset<HC>(W, r, obs);
-        walker::store_world(W, a.lunar_rec, a.n, i, r, HC);
-        pcg64_store(a.rng + 4 * i, r.g);
-        a.elapsed[i] = 0;
-        store_obs_all<24>(a, i, obs);
-    }
-}
-
-template <bool HC>
-__global__ void __launch_bounds__(kLunarThreads) walker_reset_kernel(uint32_t *rec, int32_t *elapsed, uint64_t *rng,
-                                                                     const uint8_t *mask, float *obs, int64_t n) {
-    const int64_t i = (int64_t)blockIdx.x * kLunarThreads + threadIdx.x;
-    if (i >= n) return;
-    if (mask && !mask[i]) return;
-    walker::World W;
-    walker::Rng r;
-    walker::bind_world(W, rec, n, i);
-    W.flags = rec[(int64_t)walker::W_FLAGS * n + i] & b2l::kFlagsKept;  // the b2World object survives reset()
-    r.has32 = rec[(int64_t)walker::W_RNG32 * n + i];
-    r.val32 = rec[(int64_t)(walker::W_RNG32 + 1) * n + i];
-    r.g = pcg64_load(rng + 4 * i);
-    float o[24];
-    W.np = 0; W.p_lo = 0; W.p_hi = -1;
-    walker::env_reset<HC>(W, r, o);
-    walker::store_world(W, rec, n, i, r, HC);
-    pcg64_store(rng + 4 * i, r.g);
-    elapsed[i] = 0;
-    if (obs) store_row<24>(obs, i, o);
-}
-
+// ---- BipedalWalker-v3 only ------------------------------------------------------------------------------------
 // a fresh Generator has an empty 32-bit cache: clear {has_uint32, uinteger} of the (re)seeded envs
 __global__ void walker_clear_rng32_kernel(uint32_t *rec, const uint8_t *mask, int64_t n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1339,7 +1203,7 @@ template <int KIND, typename ActT>
 static int launch_step_typed(b200gym *h, const StepArgs &a, cudaStream_t st) {
     int64_t done = 0;
     const int64_t tiles = a.count / kThreads;
-    if ((a.npeer > 0 || a.bulk_sink) && h->gather_bulk && tiles > 0) {
+    if ((a.npeer > 0 || a.bulk_sink) && tiles > 0) {
         // kernel G (bulk pushes): every destination row block must be 16-byte aligned
         auto ok = [&](const float *o, const double *r, const uint8_t *te, const uint8_t *tr) {
             return (uintptr_t)(o + a.first * Env<KIND>::D) % 16 == 0 && (uintptr_t)(r + a.first) % 16 == 0 &&
@@ -1348,15 +1212,9 @@ static int launch_step_typed(b200gym *h, const StepArgs &a, cudaStream_t st) {
         bool aligned = ok(a.obs, a.reward, a.terminated, a.truncated);
         for (int p = 0; p < a.npeer; p++) aligned = aligned && ok(a.peer_obs[p], a.peer_reward[p], a.peer_term[p], a.peer_trunc[p]);
         if (aligned) {
-            StepArgs g = a;
-            // the fused step barrier needs the whole range in this one launch (a ragged tail goes through kernel A,
-            // whose stores the barrier would not cover): otherwise b200gym_step_p2p launches p2p_sync_kernel
-            const bool fused_barrier = a.p2p_done != nullptr && tiles * kThreads == a.count;
-            if (!fused_barrier) g.p2p_done = nullptr;
-            step_kernel_gather<KIND, ActT><<<(unsigned)tiles, kThreads, 0, st>>>(g);
+            step_kernel_gather<KIND, ActT><<<(unsigned)tiles, kThreads, 0, st>>>(a);
             CK(h, cudaGetLastError());
             done = tiles * kThreads;
-            h->p2p_barrier_fused = fused_barrier;
         }
     }
     if (done == 0 && h->kernel_choice >= 1 && a.npeer == 0 && a.count >= (int64_t)h->sm_count * kThreads) {
@@ -1367,37 +1225,17 @@ static int launch_step_typed(b200gym *h, const StepArgs &a, cudaStream_t st) {
         if (aligned) {
             // the lean instantiation: no fused episode statistics, every index fits 32 bits
             const bool lean = h->kernel_choice == 2 && !a.ep_acc && h->n < (int64_t)1 << 30;
-            const bool deep = h->p_depth == 2;
-            int &occ = h->occ[KIND][sizeof(ActT) == 8 ? 0 : sizeof(ActT) == 4 ? 1 : 2][(lean ? 1 : 0) + (deep ? 2 : 0)];
+            int &occ = h->occ[KIND][sizeof(ActT) == 8 ? 0 : sizeof(ActT) == 4 ? 1 : 2][lean ? 1 : 0];
             if (occ == 0) {
-                if (lean && deep) CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, step_kernel_persistent<KIND, ActT, true, 2>, kThreads, 0));
-                else if (lean) CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, step_kernel_persistent<KIND, ActT, true, 1>, kThreads, 0));
-                else if (deep) CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, step_kernel_persistent<KIND, ActT, false, 2>, kThreads, 0));
-                else CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, step_kernel_persistent<KIND, ActT, false, 1>, kThreads, 0));
+                if (lean) CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, step_kernel_persistent<KIND, ActT, true>, kThreads, 0));
+                else CK(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, step_kernel_persistent<KIND, ActT, false>, kThreads, 0));
                 if (occ < 1) occ = 1;
             }
             const int64_t all_tiles = (a.count + kThreads - 1) / kThreads;
-            // resident CTAs per SM: the occupancy limit, or -- when that leaves the last round of tiles mostly
-            // empty -- the smaller count that makes every CTA walk (nearly) the same number of tiles
-            int per_sm = occ;
-            if (h->p_ctas > 0 && h->p_ctas < occ) per_sm = h->p_ctas;
-            else if (h->p_ctas == 0) {
-                double best = 0.0;
-                for (int c = occ; c >= (occ > 2 ? occ - 2 : 1); c--) {
-                    const int64_t g = (int64_t)h->sm_count * c;
-                    const int64_t rounds = (all_tiles + g - 1) / g;
-                    // throughput model: tiles per round-time; a round's time grows with the resident warps only
-                    // weakly (latency-bound), so weigh occupancy by its square root
-                    const double score = (double)all_tiles / (double)(rounds * g) * sqrt((double)c / occ);
-                    if (score > best + 1e-9) { best = score; per_sm = c; }
-                }
-            }
-            int64_t grid = (int64_t)h->sm_count * per_sm;
+            int64_t grid = (int64_t)h->sm_count * occ;
             if (grid > all_tiles) grid = all_tiles;
-            if (lean && deep) step_kernel_persistent<KIND, ActT, true, 2><<<(unsigned)grid, kThreads, 0, st>>>(a, (int)all_tiles);
-            else if (lean) step_kernel_persistent<KIND, ActT, true, 1><<<(unsigned)grid, kThreads, 0, st>>>(a, (int)all_tiles);
-            else if (deep) step_kernel_persistent<KIND, ActT, false, 2><<<(unsigned)grid, kThreads, 0, st>>>(a, (int)all_tiles);
-            else step_kernel_persistent<KIND, ActT, false, 1><<<(unsigned)grid, kThreads, 0, st>>>(a, (int)all_tiles);
+            if (lean) step_kernel_persistent<KIND, ActT, true><<<(unsigned)grid, kThreads, 0, st>>>(a, (int)all_tiles);
+            else step_kernel_persistent<KIND, ActT, false><<<(unsigned)grid, kThreads, 0, st>>>(a, (int)all_tiles);
             CK(h, cudaGetLastError());
             done = a.count;
         }
@@ -1406,8 +1244,7 @@ static int launch_step_typed(b200gym *h, const StepArgs &a, cudaStream_t st) {
         StepArgs t = a;
         t.first = a.first + done;
         t.count = a.count - done;
-        const int bs = h->block_a;
-        step_kernel<KIND, ActT><<<(unsigned)((t.count + bs - 1) / bs), bs, 0, st>>>(t);
+        step_kernel<KIND, ActT><<<blocks_for(t.count), kThreads, 0, st>>>(t);
         CK(h, cudaGetLastError());
     }
     return 0;
@@ -1430,6 +1267,26 @@ static int launch_step_kind(b200gym *h, const StepArgs &a, int action_dtype, cud
     }
 }
 
+// The Box2D step: box2d_step_kernel -> box2d_toi_kernel -> box2d_reset_list_kernel on the stream.  The caller may
+// have picked the counters' slot (one per concurrently running launch range).
+template <typename Step>
+static int launch_box2d_step(b200gym *h, const StepArgs &a, cudaStream_t st) {
+    using Task = typename Step::Task;
+    if (a.autoreset) CK(h, cudaMemsetAsync(a.reset_count, 0, sizeof(int32_t), st));
+    CK(h, cudaMemsetAsync(a.toi_count, 0, sizeof(int32_t), st));
+    box2d_step_kernel<Step><<<(unsigned)((a.count + kBox2dThreads - 1) / kBox2dThreads), kBox2dThreads, 0, st>>>(a);
+    CK(h, cudaGetLastError());
+    box2d_toi_kernel<Task><<<(unsigned)std::min<int64_t>(a.count, (int64_t)kToiCtasPerSm * h->sm_count), 32, 0, st>>>(a);
+    CK(h, cudaGetLastError());
+    if (a.autoreset) {
+        // at most this many CTAs (the kernel strides over the list)
+        const int64_t grid = std::min<int64_t>((a.count + kBox2dThreads - 1) / kBox2dThreads, 2 * h->sm_count);
+        box2d_reset_list_kernel<Task><<<(unsigned)grid, kBox2dThreads, 0, st>>>(a);
+        CK(h, cudaGetLastError());
+    }
+    return 0;
+}
+
 static int launch_step(b200gym *h, const StepArgs &a, int action_dtype, cudaStream_t st) {
     switch (h->cfg.kind) {
     case B200GYM_CARTPOLE: return launch_step_kind<B200GYM_CARTPOLE>(h, a, action_dtype, st);
@@ -1438,103 +1295,22 @@ static int launch_step(b200gym *h, const StepArgs &a, int action_dtype, cudaStre
     case B200GYM_PENDULUM: return launch_step_kind<B200GYM_PENDULUM>(h, a, action_dtype, st);
     case B200GYM_ACROBOT: return launch_step_kind<B200GYM_ACROBOT>(h, a, action_dtype, st);
     case B200GYM_LUNARLANDER:
+        switch (action_dtype) {
+        case B200GYM_ACT_I64: return launch_box2d_step<LunarStep<long long, false>>(h, a, st);
+        case B200GYM_ACT_I32: return launch_box2d_step<LunarStep<int, false>>(h, a, st);
+        case B200GYM_ACT_U8: return launch_box2d_step<LunarStep<unsigned char, false>>(h, a, st);
+        default: return fail(h, "Discrete env needs an integer action dtype (got code %d)", action_dtype);
+        }
     case B200GYM_LUNARLANDER_CONT:
+        if (action_dtype != B200GYM_ACT_F32) return fail(h, "Box env needs float32 actions (got dtype code %d)", action_dtype);
+        if ((uintptr_t)a.actions % 8 != 0) return fail(h, "LunarLanderContinuous actions must be 8-byte aligned");
+        return launch_box2d_step<LunarStep<float, true>>(h, a, st);
     case B200GYM_BIPEDALWALKER:
-    case B200GYM_BIPEDALWALKER_HARDCORE: {
-        StepArgs b = a;
-        const bool defer = h->cfg.autoreset && h->box2d_defer && h->reset_list;
-        if (defer) {   // the caller may have picked a counter slot (one per concurrently running range)
-            b.reset_list = h->reset_list;
-            if (!b.reset_count) b.reset_count = h->reset_count;
-            CK(h, cudaMemsetAsync(b.reset_count, 0, sizeof(int32_t), st));
-        } else {
-            b.reset_list = nullptr; b.reset_count = nullptr;
-        }
-        // continuous collision of the parked envs in its own launch (see lunar_toi_kernel)
-        const bool toi_defer = h->box2d_toi_defer && h->toi_list;
-        if (toi_defer) {
-            b.toi_list = h->toi_list;
-            b.toi_mid = h->toi_mid;
-            if (!b.toi_count) b.toi_count = h->toi_count;
-            CK(h, cudaMemsetAsync(b.toi_count, 0, sizeof(int32_t), st));
-        } else {
-            b.toi_list = nullptr; b.toi_count = nullptr; b.toi_mid = nullptr;
-        }
-        // one warp per CTA, 12 CTAs per SM (what is resident with the 156-register kernel); the kernel strides over
-        // the list.  Larger grids (fewer envs per warp) were measured: LunarLander 1.74 / 1.82 / 1.85 ms at 12 / 64 / 256
-        // CTAs per SM, BipedalWalker (nearly every env parked) 7.4 / 12.2 / 17.1 ms
-        const unsigned tgrid = (unsigned)std::min<int64_t>(b.count, (int64_t)h->toi_grid * h->sm_count);
-        // With both on, the resets come from two kernels: those of the step kernel go onto list 1 and restart on the
-        // side stream WHILE the TOI kernel runs (a reset is a long serial chain -- terrain draw + an embedded world
-        // step, 1.1 ms for a batch of BipedalWalker resets -- but touches only its own env); those of the TOI kernel
-        // go onto list 2 and restart after it.  b2 = the arguments of the TOI kernel and of the second reset launch.
-        const bool split = defer && toi_defer && h->side && h->box2d_split;
-        StepArgs b2 = b;
-        if (split) {
-            const ptrdiff_t slot = b.reset_count - h->reset_count;   // the caller's counter slot
-            b2.reset_list = h->reset_list2;
-            b2.reset_count = h->reset_count2 + ((slot >= 0 && slot < kResetSlots) ? slot : 0);
-            CK(h, cudaMemsetAsync(b2.reset_count, 0, sizeof(int32_t), st));
-        }
-        // at most this many CTAs of the compacted reset kernel (it strides over the list)
-        const unsigned rgrid = (unsigned)std::min<int64_t>((b.count + kLunarThreads - 1) / kLunarThreads, 2 * h->sm_count);
-        if (h->is_lunar) {
-            const int bs = h->box2d_block;
-            const unsigned grid = (unsigned)((b.count + bs - 1) / bs);
-            if (h->cfg.kind == B200GYM_LUNARLANDER_CONT) {
-                if (action_dtype != B200GYM_ACT_F32) return fail(h, "Box env needs float32 actions (got dtype code %d)", action_dtype);
-                if ((uintptr_t)b.actions % 8 != 0) return fail(h, "LunarLanderContinuous actions must be 8-byte aligned");
-                lunar_step_kernel<float, true><<<grid, bs, 0, st>>>(b);
-            } else {
-                switch (action_dtype) {
-                case B200GYM_ACT_I64: lunar_step_kernel<long long, false><<<grid, bs, 0, st>>>(b); break;
-                case B200GYM_ACT_I32: lunar_step_kernel<int, false><<<grid, bs, 0, st>>>(b); break;
-                case B200GYM_ACT_U8: lunar_step_kernel<unsigned char, false><<<grid, bs, 0, st>>>(b); break;
-                default: return fail(h, "Discrete env needs an integer action dtype (got code %d)", action_dtype);
-                }
-            }
-            CK(h, cudaGetLastError());
-            if (split) {   // the step kernel's resets on the side stream, under the TOI kernel
-                CK(h, cudaEventRecord(h->ev_fork, st));
-                CK(h, cudaStreamWaitEvent(h->side, h->ev_fork, 0));
-                lunar_reset_list_kernel<<<rgrid, kLunarThreads, 0, h->side>>>(b);
-                CK(h, cudaEventRecord(h->ev_join, h->side));
-            }
-            if (toi_defer) {
-                lunar_toi_kernel<<<tgrid, 32, 0, st>>>(b2);
-                CK(h, cudaGetLastError());
-            }
-            if (defer) lunar_reset_list_kernel<<<rgrid, kLunarThreads, 0, st>>>(b2);
-            if (split) CK(h, cudaStreamWaitEvent(st, h->ev_join, 0));
-        } else {
-            if (action_dtype != B200GYM_ACT_F32) return fail(h, "Box env needs float32 actions (got dtype code %d)", action_dtype);
-            if ((uintptr_t)b.actions % 16 != 0) return fail(h, "BipedalWalker actions must be 16-byte aligned");
-            const unsigned grid = (unsigned)((b.count + kLunarThreads - 1) / kLunarThreads);
-            const bool hc = h->cfg.kind == B200GYM_BIPEDALWALKER_HARDCORE;
-            if (hc) walker_step_kernel<true><<<grid, kLunarThreads, 0, st>>>(b);
-            else walker_step_kernel<false><<<grid, kLunarThreads, 0, st>>>(b);
-            CK(h, cudaGetLastError());
-            if (split) {   // the step kernel's resets on the side stream, under the TOI kernel
-                CK(h, cudaEventRecord(h->ev_fork, st));
-                CK(h, cudaStreamWaitEvent(h->side, h->ev_fork, 0));
-                if (hc) walker_reset_list_kernel<true><<<rgrid, kLunarThreads, 0, h->side>>>(b);
-                else walker_reset_list_kernel<false><<<rgrid, kLunarThreads, 0, h->side>>>(b);
-                CK(h, cudaEventRecord(h->ev_join, h->side));
-            }
-            if (toi_defer) {
-                if (hc) walker_toi_kernel<true><<<tgrid, 32, 0, st>>>(b2);
-                else walker_toi_kernel<false><<<tgrid, 32, 0, st>>>(b2);
-                CK(h, cudaGetLastError());
-            }
-            if (defer) {
-                if (hc) walker_reset_list_kernel<true><<<rgrid, kLunarThreads, 0, st>>>(b2);
-                else walker_reset_list_kernel<false><<<rgrid, kLunarThreads, 0, st>>>(b2);
-            }
-            if (split) CK(h, cudaStreamWaitEvent(st, h->ev_join, 0));
-        }
-        CK(h, cudaGetLastError());
-        return 0;
-    }
+    case B200GYM_BIPEDALWALKER_HARDCORE:
+        if (action_dtype != B200GYM_ACT_F32) return fail(h, "Box env needs float32 actions (got dtype code %d)", action_dtype);
+        if ((uintptr_t)a.actions % 16 != 0) return fail(h, "BipedalWalker actions must be 16-byte aligned");
+        if (h->cfg.kind == B200GYM_BIPEDALWALKER_HARDCORE) return launch_box2d_step<WalkerTask<true>>(h, a, st);
+        return launch_box2d_step<WalkerTask<false>>(h, a, st);
     }
     return fail(h, "bad kind %d", h->cfg.kind);
 }
@@ -1548,6 +1324,12 @@ static void launch_reset_kind(b200gym *h, const uint8_t *mask, const double *bou
                                                               h->n, lo, hi);
 }
 
+template <typename Task>
+static void launch_box2d_reset(b200gym *h, const uint8_t *mask, float *obs, cudaStream_t st) {
+    box2d_reset_kernel<Task><<<(unsigned)((h->n + kBox2dThreads - 1) / kBox2dThreads), kBox2dThreads, 0, st>>>(
+        h->lunar_rec, h->elapsed, h->rng, mask, obs, h->n, h->lunar_opts);
+}
+
 static int launch_reset(b200gym *h, const uint8_t *mask, const double *bounds, float *obs, cudaStream_t st) {
     switch (h->cfg.kind) {
     case B200GYM_CARTPOLE: launch_reset_kind<B200GYM_CARTPOLE>(h, mask, bounds, obs, st); break;
@@ -1556,18 +1338,9 @@ static int launch_reset(b200gym *h, const uint8_t *mask, const double *bounds, f
     case B200GYM_PENDULUM: launch_reset_kind<B200GYM_PENDULUM>(h, mask, bounds, obs, st); break;
     case B200GYM_ACROBOT: launch_reset_kind<B200GYM_ACROBOT>(h, mask, bounds, obs, st); break;
     case B200GYM_LUNARLANDER:
-    case B200GYM_LUNARLANDER_CONT:
-        lunar_reset_kernel<<<(unsigned)((h->n + kLunarThreads - 1) / kLunarThreads), kLunarThreads, 0, st>>>(
-            h->lunar_rec, h->elapsed, h->rng, mask, obs, h->n, h->lunar_opts);
-        break;
-    case B200GYM_BIPEDALWALKER:
-        walker_reset_kernel<false><<<(unsigned)((h->n + kLunarThreads - 1) / kLunarThreads), kLunarThreads, 0, st>>>(
-            h->lunar_rec, h->elapsed, h->rng, mask, obs, h->n);
-        break;
-    case B200GYM_BIPEDALWALKER_HARDCORE:
-        walker_reset_kernel<true><<<(unsigned)((h->n + kLunarThreads - 1) / kLunarThreads), kLunarThreads, 0, st>>>(
-            h->lunar_rec, h->elapsed, h->rng, mask, obs, h->n);
-        break;
+    case B200GYM_LUNARLANDER_CONT: launch_box2d_reset<LunarTask>(h, mask, obs, st); break;
+    case B200GYM_BIPEDALWALKER: launch_box2d_reset<WalkerTask<false>>(h, mask, obs, st); break;
+    case B200GYM_BIPEDALWALKER_HARDCORE: launch_box2d_reset<WalkerTask<true>>(h, mask, obs, st); break;
     default: return fail(h, "bad kind %d", h->cfg.kind);
     }
     CK(h, cudaGetLastError());
@@ -1628,31 +1401,8 @@ extern "C" int b200gym_create(const b200gym_config *cfg, int64_t num_envs, int d
     h->A = k_act_dim[cfg->kind];
     h->NACT = k_nact[cfg->kind];
     h->sm_count = prop.multiProcessorCount > 0 ? prop.multiProcessorCount : 148;
-    {
-        const char *fs = getenv("B200GYM_SIMPLE_KERNEL");
-        const char *kc = getenv("B200GYM_KERNEL");
-        if (kc && (kc[0] == 'a' || kc[0] == 'p' || kc[0] == 'l')) h->kernel_choice = kc[0] == 'a' ? 0 : kc[0] == 'p' ? 1 : 2;
-        const char *pd = getenv("B200GYM_P_DEPTH");
-        if (pd && (pd[0] == '1' || pd[0] == '2')) h->p_depth = pd[0] - '0';
-        const char *pc = getenv("B200GYM_P_CTAS");
-        if (pc && atoi(pc) >= -1 && atoi(pc) <= 8) h->p_ctas = atoi(pc);
-        if (fs && fs[0] == '1') h->kernel_choice = 0;
-        const char *pfb = getenv("B200GYM_P2P_FUSE_BARRIER");
-        if (pfb && (pfb[0] == '0' || pfb[0] == '1')) h->p2p_fuse = pfb[0] - '0';
-        const char *gb = getenv("B200GYM_GATHER");
-        if (gb && (gb[0] == 'b' || gb[0] == 'd')) h->gather_bulk = gb[0] == 'b';
-        const char *bb = getenv("B200GYM_BOX2D_BLOCK");
-        if (bb && (atoi(bb) == 128 || atoi(bb) == 256)) h->box2d_block = atoi(bb);
-        const char *bsp = getenv("B200GYM_BOX2D_SPLIT");
-        if (bsp && (bsp[0] == '0' || bsp[0] == '1')) h->box2d_split = bsp[0] - '0';
-        if (const char *tge = getenv("B200GYM_TOI_GRID")) { const int v = atoi(tge); if (v >= 1 && v <= 1024) h->toi_grid = v; }
-        const char *btd = getenv("B200GYM_BOX2D_TOI_DEFER");
-        if (btd && (btd[0] == '0' || btd[0] == '1')) h->box2d_toi_defer = btd[0] - '0';
-        const char *bdf = getenv("B200GYM_BOX2D_DEFER");
-        if (bdf && (bdf[0] == '0' || bdf[0] == '1')) h->box2d_defer = bdf[0] - '0';
-        const char *ba = getenv("B200GYM_BLOCK_A");
-        if (ba && (atoi(ba) == 64 || atoi(ba) == 128 || atoi(ba) == 256)) h->block_a = atoi(ba);
-    }
+    if (const char *kc = getenv("B200GYM_KERNEL"))
+        if (kc[0] == 'a' || kc[0] == 'p' || kc[0] == 'l') h->kernel_choice = kc[0] == 'a' ? 0 : kc[0] == 'p' ? 1 : 2;
     DeviceGuard guard(device);
     const size_t n = (size_t)num_envs;
     cudaError_t es[5] = {
@@ -1687,12 +1437,6 @@ extern "C" int b200gym_create(const b200gym_config *cfg, int64_t num_envs, int d
         if (cudaMalloc(&h->lunar_rec, sizeof(uint32_t) * words * n) != cudaSuccess ||
             cudaMemset(h->lunar_rec, 0, sizeof(uint32_t) * words * n) != cudaSuccess ||
             cudaMalloc((void **)&h->reset_list, sizeof(int32_t) * n) != cudaSuccess ||
-            cudaMalloc((void **)&h->reset_list2, sizeof(int32_t) * n) != cudaSuccess ||
-            cudaMalloc((void **)&h->reset_count2, sizeof(int32_t) * kResetSlots) != cudaSuccess ||
-            cudaMemset(h->reset_count2, 0, sizeof(int32_t) * kResetSlots) != cudaSuccess ||
-            cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking) != cudaSuccess ||
-            cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
-            cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming) != cudaSuccess ||
             cudaMalloc((void **)&h->toi_list, sizeof(int32_t) * n) != cudaSuccess ||
             cudaMalloc((void **)&h->toi_count, sizeof(int32_t) * kResetSlots) != cudaSuccess ||
             cudaMemset(h->toi_count, 0, sizeof(int32_t) * kResetSlots) != cudaSuccess ||
@@ -1748,17 +1492,11 @@ extern "C" void b200gym_destroy(b200gym_t *h) {
     cudaFree(h->toi_list);
     cudaFree(h->toi_count);
     cudaFree(h->toi_mid);
-    cudaFree(h->reset_list2);
-    cudaFree(h->reset_count2);
-    if (h->side) cudaStreamDestroy(h->side);
-    if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-    if (h->ev_join) cudaEventDestroy(h->ev_join);
     if (h->p2p.base) {
         for (int r = 0; r < h->p2p.world; r++)
             if (r != h->p2p.rank && h->p2p.peer[r]) cudaIpcCloseMemHandle(h->p2p.peer[r]);
         cudaFree(h->p2p.base);
         cudaFree(h->d_peer_flags);
-        cudaFree(h->p2p_done);
     }
     delete h;
 }
@@ -1820,10 +1558,8 @@ static StepArgs make_args(b200gym *h, const void *actions, float *obs, double *r
     a.n = h->n; a.first = 0; a.count = h->n;
     a.max_steps = h->cfg.max_episode_steps; a.autoreset = h->cfg.autoreset; a.param0 = h->cfg.param[0];
     a.lunar_opts = h->lunar_opts;
-    a.reset_list = nullptr; a.reset_count = nullptr;
-    a.toi_list = nullptr; a.toi_count = nullptr; a.toi_mid = nullptr;
-    a.p2p_done = nullptr; a.p2p_peer_flags = nullptr; a.p2p_my_flags = nullptr; a.p2p_timed_out = nullptr;
-    a.p2p_step = 0; a.p2p_timeout_ns = 0; a.p2p_world = 0; a.p2p_rank = 0;
+    a.reset_list = h->reset_list; a.reset_count = h->reset_count;   // Box2D tasks (null otherwise); counter slot 0
+    a.toi_list = h->toi_list; a.toi_count = h->toi_count; a.toi_mid = h->toi_mid;
     a.npeer = 0;
     a.bulk_sink = 0;
     a.ep_acc = h->ep.acc; a.ep_len = h->ep.len; a.ep_r = h->ep.r; a.ep_l = h->ep.l;
@@ -2001,19 +1737,9 @@ extern "C" int b200gym_step_p2p(b200gym_t *h, const void *actions_dev, int actio
         for (int r = 0; r < P.world; r++) pf[r] = (unsigned long long *)(P.peer[r] + P.off_flags);
         CK(h, cudaMalloc((void **)&h->d_peer_flags, sizeof pf));
         CK(h, cudaMemcpy(h->d_peer_flags, pf, sizeof pf, cudaMemcpyHostToDevice));
-        CK(h, cudaMalloc((void **)&h->p2p_done, sizeof(unsigned int)));
-        CK(h, cudaMemset(h->p2p_done, 0, sizeof(unsigned int)));
     }
-    if (P.world > 1 && h->p2p_fuse) {   // offer kernel G the step barrier (it takes it when it covers the whole range)
-        a.p2p_done = h->p2p_done;
-        a.p2p_peer_flags = h->d_peer_flags;
-        a.p2p_my_flags = (const unsigned long long *)(P.base + P.off_flags);
-        a.p2p_timed_out = (int *)(P.base + P.off_flags + 128);
-        a.p2p_step = P.step; a.p2p_timeout_ns = P.timeout_ns; a.p2p_world = P.world; a.p2p_rank = P.rank;
-    }
-    h->p2p_barrier_fused = false;
     if (launch_step(h, a, action_dtype, st)) return 1;
-    if (P.world > 1 && !h->p2p_barrier_fused) {
+    if (P.world > 1) {
         // tell every peer that my rows of step `P.step` are in its buffers, then wait for theirs
         p2p_sync_kernel<<<1, 32, 0, st>>>(h->d_peer_flags, (const unsigned long long *)(P.base + P.off_flags), P.world,
                                           P.rank, P.step, P.timeout_ns, (int *)(P.base + P.off_flags + 128));

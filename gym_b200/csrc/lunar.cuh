@@ -311,5 +311,20 @@ LD void store_world(const World &W, uint32_t *rec, int64_t n, int64_t i, bool wi
     }
 }
 
+// reset() of env i in the SoA record `rec` and the [n][4] PCG64 records `rng`.  The b2World object survives reset():
+// so do the kept flag bits and wind_idx / torque_idx.  `n` is taken by reference: a kernel that passes a field of its
+// parameter block then reads it where the record is addressed, and the compiler keeps one multiply per record row out
+// of the reset-list kernel's loop instead of re-deriving rows from each other and spilling (8 / 24 / 44 bytes)
+LD void reset_from_record(uint32_t *rec, const int64_t &n, int64_t i, uint64_t *rng, const Opts &O, float (&obs)[8]) {
+    World W;
+    W.flags = rec[(int64_t)W_FLAGS * n + i] & kFlagsKept;
+    W.wind_idx = O.wind ? (int32_t)rec[(int64_t)W_WIND * n + i] : 0;
+    W.torque_idx = O.wind ? (int32_t)rec[(int64_t)(W_WIND + 1) * n + i] : 0;
+    Pcg64 g = bgym::pcg64_load(rng + 4 * i);
+    env_reset(W, g, O, obs);
+    store_world(W, rec, n, i, O.wind != 0);
+    bgym::pcg64_store(rng + 4 * i, g);
+}
+
 #undef LD
 }  // namespace lunar

@@ -440,5 +440,22 @@ LD void store_world(const World &W, uint32_t *rec, int64_t n, int64_t i, const R
     }
 }
 
+// reset() of env i in the SoA record `rec` and the [n][4] PCG64 records `rng`.  The b2World object survives reset():
+// so do the kept flag bits and numpy's 32-bit cache.  `n` by reference: see lunar::reset_from_record
+template <bool HC>
+LD void reset_from_record(uint32_t *rec, const int64_t &n, int64_t i, uint64_t *rng, float (&obs)[24]) {
+    World W;
+    Rng r;
+    bind_world(W, rec, n, i);
+    W.flags = rec[(int64_t)W_FLAGS * n + i] & kFlagsKept;
+    r.has32 = rec[(int64_t)W_RNG32 * n + i];
+    r.val32 = rec[(int64_t)(W_RNG32 + 1) * n + i];
+    r.g = bgym::pcg64_load(rng + 4 * i);
+    W.np = 0; W.p_lo = 0; W.p_hi = -1;
+    env_reset<HC>(W, r, obs);
+    store_world(W, rec, n, i, r, HC);
+    bgym::pcg64_store(rng + 4 * i, r.g);
+}
+
 #undef LD
 }  // namespace walker

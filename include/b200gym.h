@@ -138,8 +138,9 @@ int b200gym_reset(b200gym_t *h, const uint8_t *mask_dev, const double *bounds_ho
  * Replaces: SyncVectorEnv.step_wait (gym/vector/sync_vector_env.py:135-169) =
  * for every env: TimeLimit.step (time_limit.py:39-56) around Env.step (e.g.
  * cartpole.py:130-188) and, when the episode ended and cfg.autoreset, the
- * unseeded env.reset() of the same call (:152-156).  ONE kernel launch (environment variable
- * B200GYM_BOX2D_DEFER=1, Box2D kinds only: the resets of the step run in a second, compacted launch).
+ * unseeded env.reset() of the same call (:152-156).  Classic-control kinds: ONE kernel launch.  Box2D
+ * kinds: three launches -- the step kernel, the continuous-collision (TOI) kernel over the envs whose step
+ * may contain a TOI event, and (with cfg.autoreset) the compacted resets of the envs whose episode ended.
  *   actions_dev   [n] integers of `action_dtype`, or [n][act_dim] float32
  *   obs_dev       [n][obs_dim] float32   post-autoreset observation
  *   reward_dev    [n] float64            (SyncVectorEnv._rewards dtype, :69)

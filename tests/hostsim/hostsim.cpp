@@ -1,11 +1,15 @@
 // hostsim.cpp -- the device solver source of the Box2D tasks, compiled for the CPU.
 //
 // TEST INFRASTRUCTURE (never shipped, never imported by gym_b200/): includes gym_b200/csrc/{rng,envs,b2lite,lunar,
-// walker}.cuh and box2d_consts.h through tests/hostsim/cuda_shim.h and drives them with plain loops that mirror the
-// bodies of lunar_step_kernel / walker_step_kernel / *_reset_kernel in gym_b200/csrc/b200gym.cu (same record layout,
-// same load -> env_step -> TimeLimit -> autoreset -> store sequence).  tests/test_hostsim_cpu.py compares it bit for
-// bit with the C oracle, so the `-m "not gpu"` suite exercises the code the kernels run: solver, scenes, record
-// packing, host-computed constants, numpy-compatible RNG.
+// walker}.cuh and box2d_consts.h through tests/hostsim/cuda_shim.h.  tests/test_hostsim_cpu.py compares it bit for bit
+// with the C oracle, so the `-m "not gpu"` suite exercises the code the kernels run: solver, scenes, record packing,
+// host-computed constants, numpy-compatible RNG.
+//   hs_reset calls the per-env reset body the reset kernels of gym_b200/csrc/b200gym.cu call
+//   (lunar::reset_from_record, walker::reset_from_record).
+//   hs_step drives env_step with a plain loop on the record layout of box2d_step_kernel, with SolveTOI and the
+//   autoreset inline, as the oracle does (load -> env_step -> TimeLimit -> autoreset -> store).  Its autoreset resets
+//   the in-flight World by hand: the device's autoreset (box2d_reset_list_kernel, which resets from the record) is
+//   covered in this suite only through hs_reset, not through the step.
 #include "cuda_shim.h"
 
 #include <cstdlib>
@@ -39,41 +43,9 @@ void ensure_consts() {
     g_consts_ready = true;
 }
 
-void lunar_reset_env(Sim &S, int64_t i, float *obs) {     // lunar_reset_kernel
-    lunar::World W;
-    W.flags = S.rec[(int64_t)lunar::W_FLAGS * S.n + i] & b2l::kFlagsKept;
-    W.wind_idx = S.opts.wind ? (int32_t)S.rec[(int64_t)lunar::W_WIND * S.n + i] : 0;
-    W.torque_idx = S.opts.wind ? (int32_t)S.rec[(int64_t)(lunar::W_WIND + 1) * S.n + i] : 0;
-    Pcg64 g = bgym::pcg64_load(&S.rng[4 * i]);
-    float o[8];
-    lunar::env_reset(W, g, S.opts, o);
-    lunar::store_world(W, S.rec.data(), S.n, i, S.opts.wind != 0);
-    bgym::pcg64_store(&S.rng[4 * i], g);
-    S.elapsed[i] = 0;
-    if (obs) std::memcpy(obs + 8 * i, o, sizeof o);
-}
-
-template <bool HC>
-void walker_reset_env(Sim &S, int64_t i, float *obs) {    // walker_reset_kernel<HC>
-    walker::World W;
-    walker::Rng r;
-    walker::bind_world(W, S.rec.data(), S.n, i);
-    W.flags = S.rec[(int64_t)walker::W_FLAGS * S.n + i] & b2l::kFlagsKept;
-    r.has32 = S.rec[(int64_t)walker::W_RNG32 * S.n + i];
-    r.val32 = S.rec[(int64_t)(walker::W_RNG32 + 1) * S.n + i];
-    r.g = bgym::pcg64_load(&S.rng[4 * i]);
-    W.np = 0; W.p_lo = 0; W.p_hi = -1;
-    float o[24];
-    walker::env_reset<HC>(W, r, o);
-    walker::store_world(W, S.rec.data(), S.n, i, r, HC);
-    bgym::pcg64_store(&S.rng[4 * i], r.g);
-    S.elapsed[i] = 0;
-    if (obs) std::memcpy(obs + 24 * i, o, sizeof o);
-}
-
 template <bool HC>
 void walker_step_env(Sim &S, int64_t i, const float *act, float *obs_out, double *reward, uint8_t *term, uint8_t *trunc,
-                     float *final_obs) {                  // walker_step_kernel<HC>
+                     float *final_obs) {                  // box2d_step_kernel<WalkerTask<HC>>
     const float action[4] = {act[4 * i], act[4 * i + 1], act[4 * i + 2], act[4 * i + 3]};
     walker::World W;
     walker::Rng rng;
@@ -148,10 +120,18 @@ void hs_get_wind_idx(void *h, int32_t *wind, int32_t *torque) {
 
 void hs_reset(void *h, float *obs) {
     Sim &S = *(Sim *)h;
-    for (int64_t i = 0; i < S.n; i++) {
-        if (S.lunar()) lunar_reset_env(S, i, obs);
-        else if (S.hardcore()) walker_reset_env<true>(S, i, obs);
-        else walker_reset_env<false>(S, i, obs);
+    for (int64_t i = 0; i < S.n; i++) {   // box2d_reset_kernel
+        if (S.lunar()) {
+            float o[8];
+            lunar::reset_from_record(S.rec.data(), S.n, i, S.rng.data(), S.opts, o);
+            if (obs) std::memcpy(obs + 8 * i, o, sizeof o);
+        } else {
+            float o[24];
+            if (S.hardcore()) walker::reset_from_record<true>(S.rec.data(), S.n, i, S.rng.data(), o);
+            else walker::reset_from_record<false>(S.rec.data(), S.n, i, S.rng.data(), o);
+            if (obs) std::memcpy(obs + 24 * i, o, sizeof o);
+        }
+        S.elapsed[i] = 0;
     }
 }
 
@@ -165,7 +145,7 @@ int64_t hs_step(void *h, const void *actions, float *obs_out, double *reward, ui
             else walker_step_env<false>(S, i, (const float *)actions, obs_out, reward, term, trunc, final_obs);
             continue;
         }
-        // lunar_step_kernel<ActT, CONT>
+        // box2d_step_kernel<LunarStep<ActT, CONT>>
         long long act = 0;
         float ca0 = 0.0f, ca1 = 0.0f;
         if (S.kind == 7) { ca0 = ((const float *)actions)[2 * i]; ca1 = ((const float *)actions)[2 * i + 1]; }

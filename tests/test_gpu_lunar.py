@@ -274,41 +274,41 @@ def test_wind_indices_default_to_numpy_global_generator():
 
 
 @pytest.mark.parametrize("env_id", ["LunarLander-v2", "BipedalWalkerHardcore-v3"])
-def test_compacted_autoreset_kernel_equals_inline_reset(env_id, monkeypatch):
+def test_three_launch_step_matches_oracle_and_host_path(env_id, monkeypatch):
     """The three-launch step of the Box2D tasks (step kernel -> TOI kernel over the parked envs -> compacted reset
-    kernel; the default) against the single-launch step with continuous collision and resets inline
-    (B200GYM_BOX2D_TOI_DEFER=0, B200GYM_BOX2D_DEFER=0): same results, on the device path and on the chunked host path
-    (every chunk has its own parked-env / reset counters)."""
+    kernel) bit for bit against the C oracle, which runs SolveTOI and the autoreset inline, and against the chunked
+    host path (every chunk has its own parked-env / reset counters).  Random play at this size goes through both
+    autoresets and TOI sub-steps."""
+    import os
+
     import gym_b200
     import torch
-    N, T = 3000, 220
-    monkeypatch.setenv("B200GYM_BOX2D_DEFER", "0")
-    monkeypatch.setenv("B200GYM_BOX2D_TOI_DEFER", "0")
-    inline = gym_b200.vector.make(env_id, N)
-    monkeypatch.setenv("B200GYM_BOX2D_DEFER", "1")
-    monkeypatch.setenv("B200GYM_BOX2D_TOI_DEFER", "1")
+    from oracle.oracle import OracleLunar, OracleWalker
+    N, T = 2048, 220
     monkeypatch.setenv("B200GYM_HOST_CHUNKS", "3")
-    deferred = gym_b200.vector.make(env_id, N)
+    dev = gym_b200.vector.make(env_id, N)
     host = gym_b200.vector.make(env_id, N, backend="numpy")
-    o0, _ = inline.reset(seed=9)
-    o1, _ = deferred.reset(seed=9)
-    o2, _ = host.reset(seed=9)
-    assert torch.equal(o0, o1) and np.array_equal(o0.cpu().numpy(), o2)
-    gen = torch.Generator(device="cuda").manual_seed(4)
+    orc = OracleLunar(N) if dev.discrete else OracleWalker(N, hardcore=True, max_episode_steps=dev.max_episode_steps)
+    nthreads = min(8, os.cpu_count() or 1)
+    o0, _ = dev.reset(seed=9)
+    o1, _ = host.reset(seed=9)
+    ref = orc.reset(seed=9)
+    assert np.array_equal(o0.cpu().numpy(), ref) and np.array_equal(o1, ref)
+    rng = np.random.default_rng(4)
     n_done = 0
     for t in range(T):
-        if inline.discrete:
-            a = torch.randint(0, 4, (N,), device="cuda", generator=gen)
-        else:
-            a = torch.rand((N, 4), device="cuda", generator=gen) * 2 - 1
-        r0, r1, r2 = inline.step(a), deferred.step(a), host.step(a.cpu().numpy())
+        a = rng.integers(0, 4, size=N) if dev.discrete else rng.uniform(-1, 1, (N, 4)).astype(np.float32)
+        r0, r1, r2 = dev.step(torch.as_tensor(a, device=dev.device)), host.step(a), orc.step(a, nthreads=nthreads)
         for k in range(4):
-            assert torch.equal(r0[k], r1[k]), f"step {t}, output {k}: device path"
-            assert np.array_equal(r0[k].cpu().numpy(), r2[k]), f"step {t}, output {k}: host path"
-        done = r0[2] | r0[3]
-        if bool(done.any()):
-            assert torch.equal(r0[4]["final_observation"][done], r1[4]["final_observation"][done])
+            assert np.array_equal(r0[k].cpu().numpy(), r2[k]), f"step {t}, output {k}: device path"
+            assert np.array_equal(r1[k], r2[k]), f"step {t}, output {k}: host path"
+        done = r2[2] | r2[3]
+        if done.any():
+            assert np.array_equal(r0[4]["final_observation"].cpu().numpy()[done], r2[4][done])
+            assert np.array_equal(np.stack(r1[4]["final_observation"][done]), r2[4][done])
         n_done += int(done.sum())
     assert n_done > N // 2
-    for e in (inline, deferred, host):
+    calls, events = orc.toi_stats()
+    assert events > 100 and calls > events
+    for e in (dev, host, orc):
         e.close()

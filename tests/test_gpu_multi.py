@@ -39,8 +39,6 @@ def _worker(rank, world, port, env_id, n_local, steps, q):
     try:
         import gym_b200
         from gym_b200.distributed import ShardedVectorEnv
-        if n_local % 256 == 0:   # whole tiles: also exercise the step barrier fused into kernel G's tail
-            os.environ["B200GYM_P2P_FUSE_BARRIER"] = "1"
         total = world * n_local
         rng = np.random.default_rng(0)
         full = gym_b200.vector.make(env_id, total, max_episode_steps=25)      # single-GPU reference
@@ -157,7 +155,7 @@ def test_wrappers_across_gpus():
 
 @pytest.mark.skipif(_ngpus() < 2, reason="needs at least 2 GPUs")
 # 148*256+640: full tiles through kernel G + a ragged tail through kernel A; 5000: ragged; 300*256 / 64*256: whole tiles
-# only -- with B200GYM_P2P_FUSE_BARRIER=1 (set by the worker for these) the step barrier runs in kernel G's tail
+# only, all through kernel G.  Every case ends the step with the p2p_sync_kernel barrier
 @pytest.mark.parametrize("env_id,n_local", [("CartPole-v1", 148 * 256 + 640), ("Pendulum-v1", 5000), ("CartPole-v1", 300 * 256),
                                             ("Acrobot-v1", 64 * 256)])
 @pytest.mark.timeout(300)

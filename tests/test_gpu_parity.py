@@ -323,12 +323,8 @@ def test_persistent_kernel_equals_simple_kernel(env_id, monkeypatch):
     envs = {}
     for k in ("a", "p", "l"):   # "l": the lean instantiation of kernel P (32-bit indices, no peer / episode code)
         monkeypatch.setenv("B200GYM_KERNEL", k)
-        monkeypatch.setenv("B200GYM_P_CTAS", "0" if k == "l" else "-1")   # "l" also runs the balanced grid ...
-        monkeypatch.setenv("B200GYM_P_DEPTH", "2" if k == "l" else "1")   # ... and two tiles in flight per thread
         envs[k] = gym_b200.vector.make(env_id, N, max_episode_steps=40)
     monkeypatch.delenv("B200GYM_KERNEL")
-    monkeypatch.delenv("B200GYM_P_CTAS")
-    monkeypatch.delenv("B200GYM_P_DEPTH")
     obs = {k: e.reset(seed=99)[0] for k, e in envs.items()}
     assert torch.equal(obs["a"], obs["p"]) and torch.equal(obs["a"], obs["l"])
     ea, ep, el_ = envs["a"], envs["p"], envs["l"]
